@@ -9,6 +9,10 @@ reference uses: ``trainable_variables`` / ``variables``, ``get_weights`` / ``set
   NN.compute_critic_grad  -> cacto_critic_grad                            (NeuralNetwork.py:150-178)
   NN.compute_actor_grad   -> cacto_actor_grad                             (NeuralNetwork.py:180-232)
 
+An actor whose hidden widths (conf.NH1, conf.NH2) are not 256 is an ``'actor_width'`` network: the same Keras layout and layer
+names, no transposed copy, run by the width-generic kernels of csrc/actor_width.cu (cacto_rollout_width / cacto_actor_forward_width /
+cacto_actor_grad_width) with the widths passed at run time.
+
 The regularisers the reference attaches to its layers are inert there (gradients are taken of the loss
 only, ``model.losses`` is never added: SURVEY.md quirk Q6) and are therefore not represented.
 The default critic ('sine', every conf) runs on the fused tiled kernels of csrc/update.cu; the elu / relu / sine-elu
@@ -27,12 +31,15 @@ from .environment import _as_cuda, _device
 from .ops import ops
 
 CRITIC_HIDDEN = (64, 64, 128, 128)
+ACTOR_MAX_WIDTH = 512        # CACTO_ACTOR_MAX_WIDTH (include/cacto_b200.h)
+GENERIC_MAX_WIDTH = 256      # units per layer of the generic critic kernels (csrc/mlp_generic.cu)
 
 
 class Network:
     """A dense network stored as one flat float32 block (+ its per-layer transposed copy and a gradient
-    accumulator).  kind: 'actor' (LeakyReLU 0.3), 'critic_sine', or 'critic_generic' (any layer table, ``acts`` per layer:
-    'sin' | 'elu' | 'leaky' | 'linear'; no transposed copy)."""
+    accumulator).  kind: 'actor' (LeakyReLU 0.3, hidden widths 256), 'actor_width' (the same at any hidden widths 1..512, no
+    transposed copy), 'critic_sine', or 'critic_generic' (any layer table, ``acts`` per layer: 'sin' | 'elu' | 'leaky' | 'linear';
+    no transposed copy)."""
 
     _registry = weakref.WeakValueDictionary()      # params address -> Network (apply_gradients looks the owner up); weak: GPU blocks are freed with the net
 
@@ -40,12 +47,15 @@ class Network:
         self.kind, self.ns, self.na, self.dims = kind, int(ns), int(na), list(dims)
         self.n = sum(i * o + o for i, o in zip(dims[:-1], dims[1:]))
         if acts is None:
-            acts = (['leaky'] * (len(dims) - 2) if kind == 'actor' else ['sin'] * (len(dims) - 2)) + ['linear']
+            acts = (['leaky'] * (len(dims) - 2) if self.is_actor else ['sin'] * (len(dims) - 2)) + ['linear']
         self.acts = list(acts)
         self.desc = _lib.make_mlp_desc(self.dims, self.acts)
         dev = _device()
         self.params = torch.zeros(self.n, dtype=torch.float32, device=dev)
-        if kind == 'critic_generic':
+        if kind == 'actor_width':
+            assert len(self.dims) == 4 and self.n == lib.cacto_actor_width_param_count(self.ns, self.na, self.dims[1], self.dims[2]), self.dims
+            self.params_T = None
+        elif kind == 'critic_generic':
             self.params_T = None
         else:
             expect = lib.cacto_critic_param_count(self.ns) if kind == 'critic_sine' else lib.cacto_actor_param_count(self.ns, self.na)
@@ -55,6 +65,10 @@ class Network:
         self._views = self._make_views(self.params)
         self._grad_views = self._make_views(self.grad)
         Network._registry[self.params.data_ptr()] = self
+
+    @property
+    def is_actor(self):
+        return self.kind in ('actor', 'actor_width')
 
     @property
     def is_critic(self):
@@ -95,7 +109,7 @@ class Network:
     def _keras_layer_names(self):
         """Layer names of the reference's Keras models with weights, in topological order (as in its archived .h5 files)."""
         L = len(self.dims) - 1
-        if self.kind == 'actor':
+        if self.is_actor:
             return ['dense' if l == 0 else f'dense_{l}' for l in range(L)]
         if self.kind == 'critic_sine':
             return ['sinusodial_representation_dense' if l == 0 else f'sinusodial_representation_dense_{l}' for l in range(L - 1)] + ['dense_3']
@@ -153,11 +167,15 @@ class NN:
 
     # -- model constructors ---------------------------------------------------------------------
     def create_actor(self):
-        """NeuralNetwork.py:51-63: Dense(NH1) LeakyReLU Dense(NH2) LeakyReLU Dense(na); glorot-uniform kernels, zero biases."""
+        """NeuralNetwork.py:51-63: Dense(NH1) LeakyReLU Dense(NH2) LeakyReLU Dense(na); glorot-uniform kernels, zero biases.
+        NH1 = NH2 = 256 (every reference conf) runs on the fused kernels ('actor'); any other widths in 1..512 on the width-generic
+        ones ('actor_width')."""
         c = self.conf
-        if (c.NH1, c.NH2) != (256, 256):
-            raise NotImplementedError('the fused actor kernels are specialised for NH1 = NH2 = 256 (every reference conf)')
-        net = Network('actor', c.nb_state, c.nb_action, [c.nb_state, c.NH1, c.NH2, c.nb_action])
+        nh1, nh2 = int(c.NH1), int(c.NH2)
+        if not (1 <= nh1 <= ACTOR_MAX_WIDTH and 1 <= nh2 <= ACTOR_MAX_WIDTH):
+            raise ValueError(f'actor hidden widths NH1 = {nh1}, NH2 = {nh2}: each must be in 1..{ACTOR_MAX_WIDTH}')
+        kind = 'actor' if (nh1, nh2) == (256, 256) else 'actor_width'
+        net = Network(kind, c.nb_state, c.nb_action, [c.nb_state, nh1, nh2, c.nb_action])
         w = []
         for i, o in zip(net.dims[:-1], net.dims[1:]):
             w += [_glorot(self._rng, i, o), np.zeros(o, np.float32)]
@@ -204,6 +222,9 @@ class NN:
         """NeuralNetwork.py:110-128: Dense 16, 32, NH1, NH2 each followed by LeakyReLU() (alpha 0.3), Dense(1); the
         regularisers are inert (quirks Q6, Q14)."""
         c = self.conf
+        if max(int(c.NH1), int(c.NH2)) > GENERIC_MAX_WIDTH:
+            raise ValueError(f"the 'relu' critic uses NH1 = {c.NH1}, NH2 = {c.NH2} as its widths; the generic critic kernels support at most "
+                             f'{GENERIC_MAX_WIDTH} units per layer')
         return self._generic_critic((16, 32, c.NH1, c.NH2), ['leaky'] * 4, [False] * 4)
 
     # -- forward ------------------------------------------------------------------------------
@@ -216,6 +237,9 @@ class NN:
         if NN.kind == 'actor':
             out = torch.empty((B, NN.na), dtype=torch.float32, device=x.device)
             ops.actor_forward(self._pt, NN.params, x, out)
+        elif NN.kind == 'actor_width':
+            out = torch.empty((B, NN.na), dtype=torch.float32, device=x.device)
+            ops.actor_forward_width(self._pt, NN.params, NN.dims[1], NN.dims[2], x, out)
         elif NN.kind == 'critic_generic':
             out = torch.empty((B, 1), dtype=torch.float32, device=x.device)
             check(lib.cacto_mlp_forward_generic(self._p, _lib.C.byref(NN.desc), ptr(NN.params), ptr(x), ptr(out), ptr(None), B, stream_ptr()),
@@ -275,6 +299,9 @@ class NN:
                             self.last_critic_loss)
 
     def launch_actor_grad(self, am, cm, s, term, inv_B, actions, B):
+        if am.kind == 'actor_width' and cm.kind == 'critic_sine':      # whatever the batch size: the tcgen05 engine is 256-wide only
+            ops.actor_grad_width(self._pt, am.params, am.dims[1], am.dims[2], cm.params, cm.params_T, s, term, inv_B, am.grad, actions)
+            return
         if cm.kind == 'critic_sine' and self._use_tc(B):
             ws = self._tc_workspace(B)
             ops.actor_grad_tc(self._pt, am.params, cm.params, s, term, inv_B, am.grad, actions, ws)

@@ -327,6 +327,15 @@ class RL_AC:
             raise ValueError('unknown rollout engine %r' % (engine,))
         use_actor = int(ep != 0)
         am = self.actor_model
+        if use_actor and am.kind == 'actor_width':
+            # any other hidden width than 256: the width-generic fp32 kernel, whatever the engine (the tcgen05 ones are 256-wide)
+            w1, w2 = am.dims[1], am.dims[2]
+            if states.is_cuda:
+                ops.rollout_width(self.env._pt, am.params, w1, w2, ics, hz, T_max, states, controls, flags, rewards)
+            else:                # zero-copy mode: pinned host outputs through UVA, plain C ABI
+                check(lib.cacto_rollout_width(self.env._p, ptr(am.params), w1, w2, ptr(ics), ptr(hz), T_max, ptr(states), ptr(controls), ptr(flags),
+                                              ptr(rewards), B, stream_ptr()), 'rollout_width')
+            return
         if engine in ('tc', 'tc2') and am.ns > 8 and not self.ur5_on_tc16:
             # UR5 is bound by its fp64 articulated-body dynamics, not by the actor: the fp16 kernel (which can run it: 4-slot W2 ring,
             # streamed layer 1) has one dynamics thread per rollout and 256 rollouts per SM and takes 7.04 ms for 32768 x 100 steps
@@ -395,13 +404,19 @@ class RL_AC:
             out['rewards'] = rewards
         return out
 
+    def _fp16_engine(self, ep, engine):
+        """Whether the rollouts of episode ``ep`` run on an fp16-split engine, whose range limit can flag a rollout failed."""
+        am = self.actor_model
+        return (ep != 0 and (engine or self.rollout_engine) in ('tc', 'tc2') and am.kind == 'actor'
+                and (am.ns <= 8 or self.ur5_on_tc16))
+
     def _retry_flagged(self, ep, ics, hz, T_max, states, controls, flags, rewards, engine=None):
         """The fp16-split engines ('tc', 'tc2') flag a rollout failed when a hidden activation leaves the fp16 range (+-2047
         after scaling, rollout_tc16.cu) -- a limit the reference does not have: RL.py:229-231 aborts on NaN only and trained
         actors are unbounded (SURVEY.md quirk Q11).  Flagged rollouts are therefore rolled out again on the fp32 'fma' engine and
         patched into the outputs; only rollouts that fail there too (a NaN state, as in the reference) stay flagged.
         Costs one device->host read of the failure count per call.  Returns the number of rollouts re-run."""
-        if ep == 0 or (engine or self.rollout_engine) not in ('tc', 'tc2') or (self.actor_model.ns > 8 and not self.ur5_on_tc16):
+        if not self._fp16_engine(ep, engine):
             return 0
         bad = (flags == 0).nonzero().reshape(-1)
         n = int(bad.numel())
@@ -532,7 +547,7 @@ class RL_AC:
 
     def _patch_flagged_host(self, ics_host, hz_np, ep, states_host, controls_host, flags_host, engine):
         """fp16-range failures of the 'tc' engines (see _retry_flagged): re-run on 'fma' and patch the host buffers."""
-        if ep != 0 and (engine or self.rollout_engine) in ('tc', 'tc2') and (self.actor_model.ns <= 8 or self.ur5_on_tc16):
+        if self._fp16_engine(ep, engine):
             bad = (flags_host == 0).nonzero().reshape(-1)
             if bad.numel() > 0:
                 r = self.rollout_batch(ics_host[bad], ep, horizon=hz_np[bad.numpy()], engine='fma')

@@ -126,6 +126,12 @@ _SIGNATURES = {
     'cacto_peer_export': (C.c_int, [C.c_void_p, C.c_void_p]),
     'cacto_peer_open': (C.c_int, [C.c_void_p, C.POINTER(C.c_void_p)]),
     'cacto_peer_close': (C.c_int, [C.c_void_p]),
+    'cacto_actor_width_param_count': (C.c_int64, [C.c_int32] * 4),
+    'cacto_rollout_width': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
+                                      C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    'cacto_actor_forward_width': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
+    'cacto_actor_grad_width': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32] + [C.c_void_p] * 4 + [C.c_float, C.c_void_p, C.c_void_p, C.c_int64,
+                                                                                                        C.c_void_p]),
     'cacto_actor_forward': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     'cacto_critic_forward': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     'cacto_critic_grad': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int] + [C.c_void_p] * 6 +

@@ -24,7 +24,8 @@ constexpr int GEN_NT = 256;          // threads per CTA (= max layer width)
 constexpr int GEN_MAXW = 256;        // max units per layer
 constexpr int GEN_MAXL = CACTO_MLP_MAX_LAYERS;
 constexpr int GEN_TOT = 1280;        // max total units of a network incl. its input (floats per activation array)
-constexpr int GEN_TOT_A = 640;       // ... of the actor in the actor step
+constexpr int GEN_MAXW_A = CACTO_ACTOR_MAX_WIDTH;              // max units per layer of the actor in the actor step
+constexpr int GEN_TOT_A = CACTO_MAX_NS + 2 * GEN_MAXW_A + CACTO_MAX_NA;   // ... and its max total units
 
 __device__ __forceinline__ float gen_slog(float x) { return x > 0.f ? logf(fmaxf(x, 1e-7f) + 1.f) : -logf(fmaxf(-x, 1e-7f) + 1.f); }
 __device__ __forceinline__ float gen_slog_grad(float x) { return fabsf(x) >= 1e-7f ? 1.f / (fabsf(x) + 1.f) : 0.f; }
@@ -270,18 +271,31 @@ __global__ void __launch_bounds__(GEN_NT) k_critic_grad_gen(const __grid_constan
 // ------------------------------------------------------------------------------------------ actor step
 // The per-sample environment terms (s' = Env.simulate_batch, Fu = Env.derivative_batch, dr/da) come from the batched kernels
 // the reference-facing API already has (cacto_dyn_step / cacto_dyn_derivative / cacto_reward); this kernel does the network part.
-struct GenActorSmem {
-  float Za[GEN_TOT_A], Ha[GEN_TOT_A], F1a[GEN_TOT_A], DLa[GEN_TOT_A], Ta[GEN_TOT_A];
-  float Z[GEN_TOT], H[GEN_TOT], F1[GEN_TOT], Q[GEN_TOT], G[GEN_TOT];
-};
+// Shared memory: five activation arrays of the actor (tot_a floats each) and five of the critic (tot_c each), sized at launch
+// from the two descriptors (gen_actor_smem_floats).
+__host__ __device__ __forceinline__ int gen_units(const cacto_mlp_desc& d) {
+  int u = 0;
+  for (int l = 0; l <= d.n_layers; ++l) u += d.dims[l];
+  return (u + 3) & ~3;
+}
+__host__ __device__ __forceinline__ int gen_actor_smem_floats(const cacto_mlp_desc& da, const cacto_mlp_desc& dc) {
+  return 5 * gen_units(da) + 5 * gen_units(dc);
+}
 
 __global__ void __launch_bounds__(GEN_NT) k_actor_grad_gen(const __grid_constant__ cacto_sys_params P, const __grid_constant__ cacto_mlp_desc DA,
                                                            const float* __restrict__ aw, const __grid_constant__ cacto_mlp_desc DC,
                                                            const float* __restrict__ cw, const float* __restrict__ state,
                                                            const float* __restrict__ state_next, const float* __restrict__ Fu,
                                                            const float* __restrict__ dr_da, float inv_B, float* __restrict__ grad) {
-  extern __shared__ __align__(16) unsigned char smem_raw[];
-  GenActorSmem& sm = *reinterpret_cast<GenActorSmem*>(smem_raw);
+  extern __shared__ __align__(16) float gen_smem[];
+  struct {
+    float *Za, *Ha, *F1a, *DLa, *Ta, *Z, *H, *F1, *Q, *G;
+  } sm;
+  {
+    const int ta = gen_units(DA), tc = gen_units(DC);
+    sm.Za = gen_smem; sm.Ha = sm.Za + ta; sm.F1a = sm.Ha + ta; sm.DLa = sm.F1a + ta; sm.Ta = sm.DLa + ta;
+    sm.Z = sm.Ta + ta; sm.H = sm.Z + tc; sm.F1 = sm.H + tc; sm.Q = sm.F1 + tc; sm.G = sm.Q + tc;
+  }
   const GenNet na_ = gen_net(DA), nc = gen_net(DC);
   const int64_t b = blockIdx.x;
   const int tid = threadIdx.x, ns = na_.dim[0], na = na_.dim[na_.L];
@@ -323,13 +337,13 @@ __global__ void __launch_bounds__(GEN_NT) k_actor_grad_gen(const __grid_constant
   }
 }
 
-static int gen_check_desc(const cacto_mlp_desc* d, int ns, int out_dim, int max_total = GEN_TOT) {
+static int gen_check_desc(const cacto_mlp_desc* d, int ns, int out_dim, int max_total = GEN_TOT, int max_width = GEN_MAXW) {
   if (!d) return CACTO_E_ARG;
   if (d->n_layers < 1 || d->n_layers > GEN_MAXL) return CACTO_E_SIZE;
   if (d->dims[0] != ns || (out_dim > 0 && d->dims[d->n_layers] != out_dim)) return CACTO_E_SIZE;
   int total = 0;
   for (int l = 0; l <= d->n_layers; ++l) {
-    if (d->dims[l] < 1 || d->dims[l] > GEN_MAXW) return CACTO_E_SIZE;
+    if (d->dims[l] < 1 || d->dims[l] > max_width) return CACTO_E_SIZE;
     total += d->dims[l];
   }
   if (total > max_total) return CACTO_E_SIZE;
@@ -385,13 +399,14 @@ extern "C" int cacto_actor_grad_generic(const cacto_sys_params* p, const cacto_m
                                         const float* state_next, const float* Fu, const float* dr_da, float inv_B, float* grad, int64_t B,
                                         void* stream) {
   if (!p) return CACTO_E_ARG;
-  if (int e = gen_check_desc(d_actor, p->ns, p->na, GEN_TOT_A)) return e;
+  if (int e = gen_check_desc(d_actor, p->ns, p->na, GEN_TOT_A, GEN_MAXW_A)) return e;
   if (int e = gen_check_desc(d_critic, p->ns, 1)) return e;
   if (B < 0 || B > 0x7fffffff) return CACTO_E_SIZE;
   if (B == 0) return 0;
   if (!actor_params || !critic_params || !state || !state_next || !Fu || !dr_da || !grad) return CACTO_E_ARG;
-  if (int e = gen_smem(k_actor_grad_gen, sizeof(GenActorSmem))) return e;
-  k_actor_grad_gen<<<(unsigned)B, GEN_NT, sizeof(GenActorSmem), (cudaStream_t)stream>>>(*p, *d_actor, actor_params, *d_critic, critic_params, state,
+  const size_t smem = 4u * (size_t)gen_actor_smem_floats(*d_actor, *d_critic);
+  if (int e = gen_smem(k_actor_grad_gen, smem)) return e;
+  k_actor_grad_gen<<<(unsigned)B, GEN_NT, smem, (cudaStream_t)stream>>>(*p, *d_actor, actor_params, *d_critic, critic_params, state,
                                                                                          state_next, Fu, dr_da, inv_B, grad);
   CACTO_LAUNCH_CHECK();
   return 0;

@@ -12,13 +12,14 @@ constexpr int ACTOR_H = 256;
 constexpr int CR_H1 = 64, CR_H2 = 64, CR_H3 = 128, CR_H4 = 128;
 constexpr float LEAKY_ALPHA = 0.3f;   // keras.layers.LeakyReLU() default
 
+// hidden widths h1 / h2: ACTOR_H for the fused kernels, any 1..CACTO_ACTOR_MAX_WIDTH for the width-generic ones (actor_width.cu)
 struct ActorLayout {
-  int ns, na;
+  int ns, na, h1, h2;
   int64_t W1, b1, W2, b2, W3, b3, total;
-  __host__ __device__ ActorLayout(int ns_, int na_) : ns(ns_), na(na_) {
-    W1 = 0; b1 = W1 + (int64_t)ns * ACTOR_H;
-    W2 = b1 + ACTOR_H; b2 = W2 + (int64_t)ACTOR_H * ACTOR_H;
-    W3 = b2 + ACTOR_H; b3 = W3 + (int64_t)ACTOR_H * na;
+  __host__ __device__ ActorLayout(int ns_, int na_, int h1_ = ACTOR_H, int h2_ = ACTOR_H) : ns(ns_), na(na_), h1(h1_), h2(h2_) {
+    W1 = 0; b1 = W1 + (int64_t)ns * h1;
+    W2 = b1 + h1; b2 = W2 + (int64_t)h1 * h2;
+    W3 = b2 + h2; b3 = W3 + (int64_t)h2 * na;
     total = b3 + na;
   }
 };

@@ -129,6 +129,42 @@ void rollout_tc16(const Tensor& p, const Tensor& actor, const Tensor& w2img, con
                         (int32_t*)dev(flags, at::kInt, "flags"), (double*)opt(rewards, F64, "rewards"), B, stream()), "rollout_tc16");
 }
 
+// ---- the actor at any hidden width (K1, N4, N7 of csrc/actor_width.cu)
+int64_t actor_width_count(const cacto_sys_params* P_, int64_t nh1, int64_t nh2) {
+  const int64_t n = cacto_actor_width_param_count(P_->ns, P_->na, (int32_t)nh1, (int32_t)nh2);
+  TORCH_CHECK(n > 0, "cacto: actor widths (", nh1, ", ", nh2, ") outside 1..", CACTO_ACTOR_MAX_WIDTH);
+  return n;
+}
+void rollout_width(const Tensor& p, const Tensor& actor, int64_t nh1, int64_t nh2, const Tensor& ics, const Tensor& horizon, int64_t T_max, Tensor states,
+                   Tensor controls, Tensor flags, const optional<Tensor>& rewards) {
+  const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
+  const int64_t B = rows_of(ics, P_->ns, "ics");
+  TORCH_CHECK(T_max >= 0, "cacto: T_max < 0");
+  need(actor, actor_width_count(P_, nh1, nh2), "actor");
+  need(horizon, B, "horizon"); need(states, (T_max + 1) * P_->ns * B, "states"); need(controls, T_max * P_->na * B, "controls"); need(flags, B, "flags");
+  need(rewards, (T_max + 1) * B, "rewards");
+  ok(cacto_rollout_width(P_, (const float*)dev(actor, F32, "actor"), (int32_t)nh1, (int32_t)nh2, (const double*)dev(ics, F64, "ics"),
+                         (const int32_t*)dev(horizon, at::kInt, "horizon"), (int32_t)T_max, (double*)dev(states, F64, "states"), (double*)dev(controls, F64, "controls"),
+                         (int32_t*)dev(flags, at::kInt, "flags"), (double*)opt(rewards, F64, "rewards"), B, stream()), "rollout_width");
+}
+void actor_forward_width(const Tensor& p, const Tensor& actor, int64_t nh1, int64_t nh2, const Tensor& state, Tensor out) {
+  const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
+  const int64_t B = rows_of(state, P_->ns, "state");
+  need(actor, actor_width_count(P_, nh1, nh2), "actor"); need(out, B * P_->na, "out");
+  ok(cacto_actor_forward_width(P_, (const float*)dev(actor, F32, "actor"), (int32_t)nh1, (int32_t)nh2, (const float*)dev(state, F32, "state"),
+                               (float*)dev(out, F32, "out"), B, stream()), "actor_forward_width");
+}
+void actor_grad_width(const Tensor& p, const Tensor& actor, int64_t nh1, int64_t nh2, const Tensor& critic, const Tensor& critic_T, const Tensor& state,
+                      const Tensor& term, double inv_B, Tensor grad, const optional<Tensor>& actions) {
+  const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
+  const int64_t B = rows_of(state, P_->ns, "state"), nact = actor_width_count(P_, nh1, nh2), nc = cacto_critic_param_count(P_->ns);
+  need(actor, nact, "actor"); need(grad, nact, "grad"); need(critic, nc, "critic"); need(critic_T, nc, "critic_T"); need(term, B, "term");
+  need(actions, B * P_->na, "actions");
+  ok(cacto_actor_grad_width(P_, (const float*)dev(actor, F32, "actor"), (int32_t)nh1, (int32_t)nh2, (const float*)dev(critic, F32, "critic"),
+                            (const float*)dev(critic_T, F32, "critic_T"), (const float*)dev(state, F32, "state"), (const double*)dev(term, F64, "term"), (float)inv_B,
+                            (float*)dev(grad, F32, "grad"), (float*)opt(actions, F32, "actions"), B, stream()), "actor_grad_width");
+}
+
 // ---- networks (N4, N6-N9)
 void actor_forward(const Tensor& p, const Tensor& actor, const Tensor& state, Tensor out) {
   const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
@@ -277,6 +313,11 @@ TORCH_LIBRARY(cacto, m) {
   m.def("actor_tc16_prepare(Tensor actor, int ns, int na, Tensor(a!) w2img) -> ()", actor_tc16_prepare);
   m.def("rollout_tc16(Tensor p, Tensor actor, Tensor w2img, Tensor ics, Tensor horizon, int T_max, Tensor(a!) states, Tensor(b!) controls, Tensor(c!) flags, "
         "Tensor(d!)? rewards) -> ()", rollout_tc16);
+  m.def("rollout_width(Tensor p, Tensor actor, int nh1, int nh2, Tensor ics, Tensor horizon, int T_max, Tensor(a!) states, Tensor(b!) controls, "
+        "Tensor(c!) flags, Tensor(d!)? rewards) -> ()", rollout_width);
+  m.def("actor_forward_width(Tensor p, Tensor actor, int nh1, int nh2, Tensor state, Tensor(a!) out) -> ()", actor_forward_width);
+  m.def("actor_grad_width(Tensor p, Tensor actor, int nh1, int nh2, Tensor critic, Tensor critic_T, Tensor state, Tensor term, float inv_B, Tensor(a!) grad, "
+        "Tensor(b!)? actions) -> ()", actor_grad_width);
   m.def("actor_forward(Tensor p, Tensor actor, Tensor state, Tensor(a!) out) -> ()", actor_forward);
   m.def("critic_forward(Tensor p, Tensor critic, Tensor state, Tensor(a!) value, Tensor(b!)? dV_ds) -> ()", critic_forward);
   m.def("critic_grad(Tensor p, Tensor critic, Tensor critic_T, Tensor target, float w_S, int mc, Tensor state, Tensor? state_next, Tensor prtg, Tensor? dVdx, "

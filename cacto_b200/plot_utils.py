@@ -33,8 +33,11 @@ class PLOT:
         controls = torch.empty((T, na, B), dtype=torch.float64, device=dev)
         flags = torch.empty(B, dtype=torch.int32, device=dev)
         rewards = torch.empty((T + 1, B), dtype=torch.float64, device=dev)
-        # the fp32 CUDA-core engine: a handful of rollouts, no fp16 range limit
-        ops.rollout(self.env._pt, actor_model.params, 1, ics, hz, T, states, controls, flags, rewards)
+        # the fp32 CUDA-core engines: a handful of rollouts, no fp16 range limit
+        if actor_model.kind == 'actor_width':
+            ops.rollout_width(self.env._pt, actor_model.params, actor_model.dims[1], actor_model.dims[2], ics, hz, T, states, controls, flags, rewards)
+        else:
+            ops.rollout(self.env._pt, actor_model.params, 1, ics, hz, T, states, controls, flags, rewards)
         per_rollout = states.permute(2, 0, 1).contiguous()                       # [B, T+1, ns]
         p_ee = torch.empty((B * (T + 1), 3), dtype=torch.float64, device=dev)
         ops.ee_position(self.env._pt, 0, per_rollout.reshape(-1, ns), p_ee)

@@ -171,9 +171,9 @@ int cacto_host_mt19937_random(uint32_t* state625, double* out, int64_t n);
 
 /* ---- Generic dense networks: the critic variants of NeuralNetwork.py besides 'sine' (create_critic_elu :65-78,
  *      create_critic_sine_elu :80-93, create_critic_relu :110-128), or any stack of <= CACTO_MLP_MAX_LAYERS dense layers of
- *      <= 256 units.  Parameter block in Keras order [W1 (in x out), b1, ...]; act[l] is the activation after layer l (the last
- *      one CACTO_ACT_LINEAR).  One CTA per sample (latency-oriented); same semantics, arguments and outputs as
- *      cacto_critic_forward / cacto_critic_grad / cacto_actor_grad, without the transposed parameter copies. */
+ *      <= 256 units (the actor of cacto_actor_grad_generic: <= CACTO_ACTOR_MAX_WIDTH units).  Parameter block in Keras order
+ *      [W1 (in x out), b1, ...]; act[l] is the activation after layer l (the last one CACTO_ACT_LINEAR).  One CTA per sample
+ *      (latency-oriented); same semantics, arguments and outputs as cacto_critic_forward / cacto_critic_grad / cacto_actor_grad, without the transposed parameter copies. */
 #define CACTO_MLP_MAX_LAYERS 8
 enum { CACTO_ACT_LINEAR = 0, CACTO_ACT_SIN = 1, CACTO_ACT_ELU = 2, CACTO_ACT_LEAKY = 3 };
 typedef struct cacto_mlp_desc {
@@ -202,6 +202,25 @@ int cacto_actor_tc16p_prepare(const float* actor_params, int32_t ns, int32_t na,
 int cacto_rollout_tc16p(const cacto_sys_params* p, const float* actor_params, const void* w2img, const double* ics,
                         const int32_t* horizon, int32_t T_max, double* states, double* controls, int32_t* flags,
                         double* rewards, int64_t B, void* stream);
+
+/* ---- The actor at any hidden width (conf.NH1 / conf.NH2; NeuralNetwork.py:51-63: ns -> nh1 -> nh2 -> na, LeakyReLU(0.3)),
+ *      1 <= nh1, nh2 <= CACTO_ACTOR_MAX_WIDTH, on fp32 CUDA-core kernels that take the widths at run time (csrc/actor_width.cu).
+ *      actor_params: the Keras-layout block of cacto_actor_width_param_count(ns, na, nh1, nh2) floats, 16-byte aligned; no
+ *      transposed or prepared copy.  cacto_actor_width_param_count returns CACTO_E_SIZE for widths out of range.
+ *      cacto_rollout_width: the contract of cacto_rollout with use_actor = 1 (RL.py:197-233; outputs may be pinned host memory).
+ *      cacto_actor_forward_width: the contract of cacto_actor_forward (NeuralNetwork.py:130-138).
+ *      cacto_actor_grad_width: the contract of cacto_actor_grad with the 'sine' critic (NeuralNetwork.py:180-232), one launch;
+ *      grad is accumulated into. */
+#define CACTO_ACTOR_MAX_WIDTH 512
+int64_t cacto_actor_width_param_count(int32_t ns, int32_t na, int32_t nh1, int32_t nh2);
+int cacto_rollout_width(const cacto_sys_params* p, const float* actor_params, int32_t nh1, int32_t nh2, const double* ics,
+                        const int32_t* horizon, int32_t T_max, double* states, double* controls, int32_t* flags, double* rewards,
+                        int64_t B, void* stream);
+int cacto_actor_forward_width(const cacto_sys_params* p, const float* actor_params, int32_t nh1, int32_t nh2, const float* state,
+                              float* out, int64_t B, void* stream);
+int cacto_actor_grad_width(const cacto_sys_params* p, const float* actor_params, int32_t nh1, int32_t nh2, const float* critic_params,
+                           const float* critic_params_T, const float* state, const double* term, float inv_B, float* grad,
+                           float* actions /* [B][na] or NULL */, int64_t B, void* stream);
 
 /* ---- N4: NN.eval over a batch (NeuralNetwork.py:130-138): out[B][na] (actor) / out[B][1] (critic) */
 int cacto_actor_forward(const cacto_sys_params* p, const float* actor_params, const float* state, float* out,
