@@ -23,6 +23,8 @@ from .optim import Adam, PiecewiseConstantDecay
 from .parallel import PeerReduce, PeerRegion, PeerUnavailable, allreduce_sum
 from .rtg import rtg_batch as _rtg_batch
 
+TC16_MAX_NS = 8          # inputs the fp16 rollout kernel holds: T16_MAX_NS = 8 in csrc/rollout_tc16.cu
+
 
 class CompactRollouts:
     """The reference-shaped view of a ``rollout_to_host(..., compact=True)`` batch: ``states(b)`` -> [T_b+1, ns] float64 with the
@@ -317,33 +319,38 @@ class RL_AC:
     # Rollout engines: 'tc' = tcgen05 fp16-split persistent kernel (cacto_rollout_tc16, default), 'tf32' = tcgen05 3xTF32
     # kernel (cacto_rollout_tc), 'fma' = fp32 CUDA-core kernel (cacto_rollout; also runs the ep = 0 zero-control rollouts).
     rollout_engine = 'tc'
-    ur5_on_tc16 = False
     use_update_graph = True          # learn_and_update replays a captured update (RL.UpdateGraph) instead of launching it eagerly
     use_pipelined_updates = True     # ... and, on one GPU, overlaps consecutive updates (RL.PipelinedUpdateGraph)
 
-    def _launch_rollout(self, ep, ics, hz, T_max, states, controls, flags, rewards, B, engine=None, prepare=True):
+    def _rollout_kernel(self, ep, engine=None):
+        """The kernel that runs the rollouts of episode ``ep`` on ``engine`` (default: ``rollout_engine``): 'fma' for the
+        zero-control rollouts of ep = 0; 'width' (cacto_rollout_width) for an actor whose hidden widths are not 256, whatever
+        the engine (the tcgen05 kernels are 256-wide); 'tf32' for 'tc' when the system has more inputs than the fp16 kernel
+        holds (UR5: its fp64 dynamics, not the actor, bound the time there, and the 3xTF32 kernel is the faster one,
+        profiles/README.md); otherwise the engine itself."""
         engine = engine or self.rollout_engine
-        if engine not in ('tc', 'tc2', 'tf32', 'fma'):
+        if engine not in ('tc', 'tf32', 'fma'):
             raise ValueError('unknown rollout engine %r' % (engine,))
+        if ep == 0:
+            return 'fma'
+        if self.actor_model.kind == 'actor_width':
+            return 'width'
+        if engine == 'tc' and self.actor_model.ns > TC16_MAX_NS:
+            return 'tf32'
+        return engine
+
+    def _launch_rollout(self, ep, ics, hz, T_max, states, controls, flags, rewards, B, engine=None, prepare=True):
+        kernel = self._rollout_kernel(ep, engine)
         use_actor = int(ep != 0)
         am = self.actor_model
-        if use_actor and am.kind == 'actor_width':
-            # any other hidden width than 256: the width-generic fp32 kernel, whatever the engine (the tcgen05 ones are 256-wide)
+        if kernel == 'width':
             w1, w2 = am.dims[1], am.dims[2]
             if states.is_cuda:
                 ops.rollout_width(self.env._pt, am.params, w1, w2, ics, hz, T_max, states, controls, flags, rewards)
             else:                # zero-copy mode: pinned host outputs through UVA, plain C ABI
                 check(lib.cacto_rollout_width(self.env._p, ptr(am.params), w1, w2, ptr(ics), ptr(hz), T_max, ptr(states), ptr(controls), ptr(flags),
                                               ptr(rewards), B, stream_ptr()), 'rollout_width')
-            return
-        if engine in ('tc', 'tc2') and am.ns > 8 and not self.ur5_on_tc16:
-            # UR5 is bound by its fp64 articulated-body dynamics, not by the actor: the fp16 kernel (which can run it: 4-slot W2 ring,
-            # streamed layer 1) has one dynamics thread per rollout and 256 rollouts per SM and takes 7.04 ms for 32768 x 100 steps
-            # against 5.62 ms of the 3xTF32 kernel (profiles/README.md), so 'tc' means the latter for UR5 unless ur5_on_tc16 is set
-            engine = 'tf32'
-        elif engine == 'tc2' and am.ns > 8:
-            engine = 'tc'
-        if use_actor and engine == 'tc':
+        elif kernel == 'tc':
             img = getattr(self, '_w2img16', None)
             if img is None:
                 img = torch.empty(int(lib.cacto_actor_tc16_image_bytes()), dtype=torch.uint8, device=am.params.device)
@@ -355,16 +362,7 @@ class RL_AC:
             else:                # zero-copy mode: the outputs are pinned HOST buffers addressed through UVA (no torch CUDA tensor): plain C ABI
                 check(lib.cacto_rollout_tc16(self.env._p, ptr(am.params), ptr(img), ptr(ics), ptr(hz), T_max, ptr(states), ptr(controls), ptr(flags),
                                              ptr(rewards), B, stream_ptr()), 'rollout_tc16')
-        elif use_actor and engine == 'tc2':
-            img = getattr(self, '_w2img16p', None)
-            if img is None:
-                img = torch.empty(int(lib.cacto_actor_tc16p_image_bytes()), dtype=torch.uint8, device=am.params.device)
-                self._w2img16p = img
-            if prepare:
-                check(lib.cacto_actor_tc16p_prepare(ptr(am.params), am.ns, am.na, ptr(img), stream_ptr()), 'actor_tc16p_prepare')
-            check(lib.cacto_rollout_tc16p(self.env._p, ptr(am.params), ptr(img), ptr(ics), ptr(hz), T_max, ptr(states), ptr(controls), ptr(flags),
-                                          ptr(rewards), B, stream_ptr()), 'rollout_tc16p')
-        elif use_actor and engine == 'tf32':
+        elif kernel == 'tf32':
             img = getattr(self, '_w2img', None)
             if img is None:
                 img = torch.empty(int(lib.cacto_actor_tc_image_floats()), dtype=torch.float32, device=am.params.device)
@@ -404,19 +402,13 @@ class RL_AC:
             out['rewards'] = rewards
         return out
 
-    def _fp16_engine(self, ep, engine):
-        """Whether the rollouts of episode ``ep`` run on an fp16-split engine, whose range limit can flag a rollout failed."""
-        am = self.actor_model
-        return (ep != 0 and (engine or self.rollout_engine) in ('tc', 'tc2') and am.kind == 'actor'
-                and (am.ns <= 8 or self.ur5_on_tc16))
-
     def _retry_flagged(self, ep, ics, hz, T_max, states, controls, flags, rewards, engine=None):
-        """The fp16-split engines ('tc', 'tc2') flag a rollout failed when a hidden activation leaves the fp16 range (+-2047
+        """The fp16-split kernel ('tc') flags a rollout failed when a hidden activation leaves the fp16 range (+-2047
         after scaling, rollout_tc16.cu) -- a limit the reference does not have: RL.py:229-231 aborts on NaN only and trained
         actors are unbounded (SURVEY.md quirk Q11).  Flagged rollouts are therefore rolled out again on the fp32 'fma' engine and
         patched into the outputs; only rollouts that fail there too (a NaN state, as in the reference) stay flagged.
         Costs one device->host read of the failure count per call.  Returns the number of rollouts re-run."""
-        if not self._fp16_engine(ep, engine):
+        if self._rollout_kernel(ep, engine) != 'tc':
             return 0
         bad = (flags == 0).nonzero().reshape(-1)
         n = int(bad.numel())
@@ -546,8 +538,8 @@ class RL_AC:
         return hz_np if wait else self._PendingRollouts(None, hz_np)
 
     def _patch_flagged_host(self, ics_host, hz_np, ep, states_host, controls_host, flags_host, engine):
-        """fp16-range failures of the 'tc' engines (see _retry_flagged): re-run on 'fma' and patch the host buffers."""
-        if self._fp16_engine(ep, engine):
+        """fp16-range failures of the 'tc' kernel (see _retry_flagged): re-run on 'fma' and patch the host buffers."""
+        if self._rollout_kernel(ep, engine) == 'tc':
             bad = (flags_host == 0).nonzero().reshape(-1)
             if bad.numel() > 0:
                 r = self.rollout_batch(ics_host[bad], ep, horizon=hz_np[bad.numpy()], engine='fma')

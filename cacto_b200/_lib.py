@@ -114,10 +114,6 @@ _SIGNATURES = {
     'cacto_critic_grad_generic': (C.c_int, [C.c_void_p] * 4 + [C.c_float, C.c_int] + [C.c_void_p] * 6 + [C.c_float] + [C.c_void_p] * 5 +
                                   [C.c_int64, C.c_void_p]),
     'cacto_actor_grad_generic': (C.c_int, [C.c_void_p] * 9 + [C.c_float, C.c_void_p, C.c_int64, C.c_void_p]),
-    'cacto_actor_tc16p_image_bytes': (C.c_int64, []),
-    'cacto_actor_tc16p_prepare': (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_void_p]),
-    'cacto_rollout_tc16p': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p,
-                                      C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),
     'cacto_adam_step_peer': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_int32, C.c_void_p, C.c_int64, C.c_void_p,
                                        C.c_void_p, C.c_void_p, C.c_float, C.c_float, C.c_float, C.c_void_p, C.c_float, C.c_void_p, C.c_int32,
                                        C.c_int32, C.c_int32, C.c_int64, C.c_int32, C.c_void_p]),

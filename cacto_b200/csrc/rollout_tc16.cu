@@ -9,6 +9,8 @@
 // [2^13, 2^14) so that the low parts stay fp16-normal; the epilogue multiplies the accumulator by 1 / (S_a S_w).
 // Range limit of this engine: a hidden activation beyond +-2047 overflows its fp16 high part -> the action becomes
 // non-finite -> the rollout is flagged failed (success = 0); the 'fma' engine has no such limit.
+// Systems: the five with at most 8 inputs and 3 actions (single / double integrator, car, car_park, manipulator); UR5
+// (13 inputs, 6 actions) runs on the 3xTF32 kernel of rollout_tc.cu, where its fp64 dynamics, not the actor, set the time.
 //
 // One persistent CTA per SM owns a contiguous range of 128-rollout tiles and runs two independent tile pipelines
 // ("slots") that share the tensor pipe and one W2 stream:
@@ -26,7 +28,7 @@
 //   warp 8 / 9       MMA issuer of slot 0 / 1 (one lane): 3 x tcgen05.mma M128 N256 K16 per chunk; tcgen05.commit
 //                    recycles the A stage, publishes the accumulator and releases the W2 ring slot.
 //   warp 10          TMA producer (one lane): streams the pre-split W2 image (16 chunks x 16 KB) from L2 into a
-//                    TC16_RING-slot ring with cp.async.bulk; both slots consume every chunk.
+//                    T16_RING-slot ring with cp.async.bulk; both slots consume every chunk.
 // Slot 1 starts its steps 8 chunks (half a step) after slot 0 -- its K-chunks are visited in the rotated order
 // 8..15,0..7, accumulation is commutative -- so that the epilogue + dynamics of one slot overlaps the MMAs of the other.
 #include <cuda_fp16.h>
@@ -50,22 +52,21 @@ constexpr int T16_B_IMG = ACTOR_H * T16_KC * 2;    // bytes of one W2 image (hi 
 constexpr int T16_IMG_BYTES = T16_NCHUNK * 2 * T16_B_IMG;   // 256 KB
 constexpr int T16_TRAILER = 64;                    // [0] u32 max|W2| bits, [1] f32 1/(S_a S_w), [2] f32 S_w
 constexpr int T16_MAXT = 512;                      // tiles per CTA that the per-tile horizon table holds
+constexpr int T16_MAX_NS = 8;                      // inputs a row publishes in the state exchange (layer-1 register tile)
+constexpr int T16_MAX_NA = 3;                      // actions the epilogue's head table holds
 constexpr float T16_SA = 32.f;
 
 template <int NS>
 struct Tc16Smem {
-  // UR5 (13 inputs: 13 KB of W1, 16 KB of state exchange) keeps a 4-slot W2 ring so that everything fits in 227 KB
-  static constexpr int RING = NS > 8 ? T16_RING / 2 : T16_RING, XW = NS > 8 ? 16 : 8;
-  alignas(1024) unsigned char B[RING][2 * T16_B_IMG];                  // W2 ring: [slot][hi | lo]           144 KB
-  alignas(1024) unsigned char A[T16_SLOTS][T16_STAGES][2 * T16_A_IMG]; // A stages: [slot][stage][hi | lo]    48 KB
-  alignas(16) float W1[NS][ACTOR_H];                                   // S_a * W1                           7-13 KB
+  alignas(1024) unsigned char B[T16_RING][2 * T16_B_IMG];              // W2 ring: [slot][hi | lo]           128 KB
+  alignas(1024) unsigned char A[T16_SLOTS][T16_STAGES][2 * T16_A_IMG]; // A stages: [slot][stage][hi | lo]    64 KB
+  alignas(16) float W1[NS][ACTOR_H];                                   // S_a * W1                           3-7 KB
   alignas(16) float b1[ACTOR_H];                                       // S_a * b1
   alignas(16) float head[ACTOR_H / 2][8];   // per column pair (c, c+1): b2 | W3[.][0] | W3[.][1] | W3[.][2]    4 KB
-  alignas(16) float headx[ACTOR_H / 2][8];  // W3[.][3] | W3[.][4] | W3[.][5] | 0 (UR5)                         4 KB
-  alignas(16) float4 xn[T16_SLOTS][XW / 4][T16_TILE];                  // normalised fp32 states of the step (row -> layer-1 threads) 8-16 KB
+  alignas(16) float4 xn[T16_SLOTS][T16_MAX_NS / 4][T16_TILE];          // normalised fp32 states of the step (row -> layer-1 threads) 8 KB
   float b3[8];
   // the issuer handles K-chunks in pairs: W2 ring slots and A stages are released (and W2 is loaded) two at a time
-  uint64_t b_full[RING / 2], b_empty[RING / 2];
+  uint64_t b_full[T16_RING / 2], b_empty[T16_RING / 2];
   uint64_t a_full[T16_SLOTS][T16_STAGES], a_empty[T16_SLOTS][T16_STAGES / 2], d_full[T16_SLOTS], start1;
   uint32_t tmem_base;
   int tile_tmax[T16_MAXT];
@@ -232,10 +233,10 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
                                                                  double* __restrict__ rewards, int64_t B, int ntiles) {
   constexpr int NX = SysDims<SYS>::NX, NA = SysDims<SYS>::NA, NS = NX + 1;
   constexpr int WORKERS = T16_WORKERS, THREADS = T16_THREADS;
-  static_assert(NS <= 16, "the layer-1 register tile holds at most 16 inputs");
+  static_assert(NS <= T16_MAX_NS, "the state exchange and the layer-1 register tile hold at most 8 inputs");
+  static_assert(NA <= T16_MAX_NA, "the epilogue's head table holds at most 3 actions");
   using Smem = Tc16Smem<NS>;
-  constexpr int RING = Smem::RING;
-  static_assert(T16_NCHUNK % T16_STAGES == 0 && T16_NCHUNK % RING == 0 && T16_HALF % RING == 0, "compile-time stage / ring indices");
+  static_assert(T16_NCHUNK % T16_STAGES == 0 && T16_NCHUNK % T16_RING == 0 && T16_HALF % T16_RING == 0, "compile-time stage / ring indices");
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   Smem& sm = *reinterpret_cast<Smem*>(smem_raw);
   const ActorLayout L(NS, NA);
@@ -250,18 +251,14 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
   for (int c = tid; c < ACTOR_H; c += THREADS) {
     sm.b1[c] = T16_SA * actor[L.b1 + c];
     float* h = &sm.head[c >> 1][c & 1];
-    float* hx = &sm.headx[c >> 1][c & 1];
     h[0] = actor[L.b2 + c];
 #pragma unroll
     for (int j = 0; j < 3; ++j) h[2 + 2 * j] = (j < NA) ? actor[L.W3 + c * NA + j] : 0.f;
-#pragma unroll
-    for (int j = 3; j < 6; ++j) hx[2 * (j - 3)] = (j < NA) ? actor[L.W3 + c * NA + j] : 0.f;
-    hx[6] = 0.f;
   }
   if (tid < 8) sm.b3[tid] = tid < NA ? actor[L.b3 + tid] : 0.f;
   for (int i = tid; i < my_tiles; i += THREADS) sm.tile_tmax[i] = 0;
   if (tid == 0) {
-    for (int s = 0; s < RING / 2; ++s) { t16_mbar_init(&sm.b_full[s], 1); t16_mbar_init(&sm.b_empty[s], 2); }
+    for (int s = 0; s < T16_RING / 2; ++s) { t16_mbar_init(&sm.b_full[s], 1); t16_mbar_init(&sm.b_empty[s], 2); }
     for (int m = 0; m < T16_SLOTS; ++m) {
       for (int s = 0; s < T16_STAGES; ++s) t16_mbar_init(&sm.a_full[m][s], T16_TILE / 2);
       for (int s = 0; s < T16_STAGES / 2; ++s) t16_mbar_init(&sm.a_empty[m][s], 1);
@@ -333,20 +330,20 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
         WEV(1);                                  // step start
         // ---- publish the normalised state of my row, fetch those of my four layer-1 rows
         {
-          float xo[16];
+          float xo[T16_MAX_NS];
 #pragma unroll
-          for (int j = 0; j < 16; ++j) xo[j] = 0.f;
+          for (int j = 0; j < T16_MAX_NS; ++j) xo[j] = 0.f;
 #pragma unroll
           for (int j = 0; j < NS; ++j) xo[j] = live ? normalize_component(P, j, (float)x[j]) : 0.f;
 #pragma unroll
-          for (int v = 0; v < Smem::XW / 4; ++v) sm.xn[m][v][row] = make_float4(xo[4 * v], xo[4 * v + 1], xo[4 * v + 2], xo[4 * v + 3]);
+          for (int v = 0; v < T16_MAX_NS / 4; ++v) sm.xn[m][v][row] = make_float4(xo[4 * v], xo[4 * v + 1], xo[4 * v + 2], xo[4 * v + 3]);
         }
         asm volatile("bar.sync %0, 128;" ::"r"(1 + m) : "memory");
         float xn[4][NS];
 #pragma unroll
         for (int i = 0; i < 4; ++i) {
 #pragma unroll
-          for (int v = 0; v < Smem::XW / 4; ++v) {
+          for (int v = 0; v < T16_MAX_NS / 4; ++v) {
             const float4 f = sm.xn[m][v][lane + 32 * i];
             if (4 * v + 0 < NS) xn[i][(4 * v + 0) % NS] = f.x;
             if (4 * v + 1 < NS) xn[i][(4 * v + 1) % NS] = f.y;
@@ -378,48 +375,26 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
             *reinterpret_cast<uint4*>(dst + 512 * i) = make_uint4(hi[0], hi[1], hi[2], hi[3]);
             *reinterpret_cast<uint4*>(dst + 512 * i + T16_A_IMG) = make_uint4(lo[0], lo[1], lo[2], lo[3]);
           };
-          if constexpr (NS <= 8) {
-            // all of W1's chunk columns in registers (8 registers per input), rows one after the other
-            ulonglong2 wA[NS], wB[NS];
+          // all of W1's chunk columns in registers (8 registers per input), rows one after the other
+          ulonglong2 wA[NS], wB[NS];
+#pragma unroll
+          for (int j = 0; j < NS; ++j) {
+            wA[j] = *reinterpret_cast<const ulonglong2*>(&sm.W1[j][c]);
+            wB[j] = *reinterpret_cast<const ulonglong2*>(&sm.W1[j][c + 4]);
+          }
+          WEV(2);                                  // chunk: W1 loaded, about to wait for the stage
+          if (qc >= T16_STAGES) t16_mbar_wait(&sm.a_empty[m][st >> 1], (uint32_t)((qc / T16_STAGES - 1) & 1));   // stage pair (st >> 1) of chunk pair qc / 2
+          WEV(3);                                  // stage free
+#pragma unroll
+          for (int i = 0; i < 4; ++i) {
+            uint64_t z[4] = {bA.x, bA.y, bB.x, bB.y};
 #pragma unroll
             for (int j = 0; j < NS; ++j) {
-              wA[j] = *reinterpret_cast<const ulonglong2*>(&sm.W1[j][c]);
-              wB[j] = *reinterpret_cast<const ulonglong2*>(&sm.W1[j][c + 4]);
+              const uint64_t xj = pk(xn[i][j], xn[i][j]);
+              z[0] = fma2(xj, wA[j].x, z[0]); z[1] = fma2(xj, wA[j].y, z[1]);
+              z[2] = fma2(xj, wB[j].x, z[2]); z[3] = fma2(xj, wB[j].y, z[3]);
             }
-            WEV(2);                                // chunk: W1 loaded, about to wait for the stage
-            if (qc >= T16_STAGES) t16_mbar_wait(&sm.a_empty[m][st >> 1], (uint32_t)((qc / T16_STAGES - 1) & 1));   // stage pair (st >> 1) of chunk pair qc / 2
-            WEV(3);                                // stage free
-#pragma unroll
-            for (int i = 0; i < 4; ++i) {
-              uint64_t z[4] = {bA.x, bA.y, bB.x, bB.y};
-#pragma unroll
-              for (int j = 0; j < NS; ++j) {
-                const uint64_t xj = pk(xn[i][j], xn[i][j]);
-                z[0] = fma2(xj, wA[j].x, z[0]); z[1] = fma2(xj, wA[j].y, z[1]);
-                z[2] = fma2(xj, wB[j].x, z[2]); z[3] = fma2(xj, wB[j].y, z[3]);
-              }
-              finish_row(i, z);
-            }
-          } else {
-            // wide inputs (UR5: 13): inputs outermost, the 4 rows' accumulators stay live (32 registers) and W1 streams through
-            uint64_t z[4][4];
-#pragma unroll
-            for (int i = 0; i < 4; ++i) { z[i][0] = bA.x; z[i][1] = bA.y; z[i][2] = bB.x; z[i][3] = bB.y; }
-#pragma unroll
-            for (int j = 0; j < NS; ++j) {
-              const ulonglong2 wa = *reinterpret_cast<const ulonglong2*>(&sm.W1[j][c]), wb = *reinterpret_cast<const ulonglong2*>(&sm.W1[j][c + 4]);
-#pragma unroll
-              for (int i = 0; i < 4; ++i) {
-                const uint64_t xj = pk(xn[i][j], xn[i][j]);
-                z[i][0] = fma2(xj, wa.x, z[i][0]); z[i][1] = fma2(xj, wa.y, z[i][1]);
-                z[i][2] = fma2(xj, wb.x, z[i][2]); z[i][3] = fma2(xj, wb.y, z[i][3]);
-              }
-            }
-            WEV(2);
-            if (qc >= T16_STAGES) t16_mbar_wait(&sm.a_empty[m][st >> 1], (uint32_t)((qc / T16_STAGES - 1) & 1));
-            WEV(3);
-#pragma unroll
-            for (int i = 0; i < 4; ++i) finish_row(i, z[i]);
+            finish_row(i, z);
           }
 #ifndef T16_EXP_NO_FENCE      // timing experiment only
           asm volatile("fence.proxy.async.shared::cta;" ::: "memory");     // generic-proxy stores -> visible to the UMMA (async proxy)
@@ -449,11 +424,6 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
             const int pair = (c0 + 8 * k) / 2 + l3;
             const ulonglong2 hA = *reinterpret_cast<const ulonglong2*>(&sm.head[pair][0]);   // b2 pair | W3[.][0] pair
             const ulonglong2 hB = *reinterpret_cast<const ulonglong2*>(&sm.head[pair][4]);   // W3[.][1] pair | W3[.][2] pair
-            ulonglong2 xA, xB;
-            if (NA > 3) {
-              xA = *reinterpret_cast<const ulonglong2*>(&sm.headx[pair][0]);
-              xB = *reinterpret_cast<const ulonglong2*>(&sm.headx[pair][4]);
-            }
 #pragma unroll
             for (int i = 0; i < 4; ++i) {                                     // row l4 + 8 i: half hl = i / 2, row half rh = i % 2
               const uint32_t* r = &v[i >> 1][4 * k + 2 * (i & 1)];
@@ -465,11 +435,6 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
               acc2[i][0] = fma2(hv, hA.y, acc2[i][0]);
               if (NA > 1) acc2[i][1] = fma2(hv, hB.x, acc2[i][1]);
               if (NA > 2) acc2[i][2] = fma2(hv, hB.y, acc2[i][2]);
-              if (NA > 3) {
-                acc2[i][3] = fma2(hv, xA.x, acc2[i][3]);
-                if (NA > 4) acc2[i][4] = fma2(hv, xA.y, acc2[i][4]);
-                if (NA > 5) acc2[i][5] = fma2(hv, xB.x, acc2[i][5]);
-              }
             }
           }
         };
@@ -552,14 +517,14 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
     constexpr uint32_t lboA = (T16_TILE / 8) * 128, lboB = (ACTOR_H / 8) * 128;
     const uint32_t d = tmem + (uint32_t)(m * ACTOR_H);
     const uint32_t a_base = smem_u32(&sm.A[m][0][0]), b_base = smem_u32(&sm.B[0][0]);
-    const uint32_t pb0 = (uint32_t)(gb / RING) & 1u;             // ring phase of this slot's first chunk (gb is 0 or T16_HALF, a multiple of RING)
+    const uint32_t pb0 = (uint32_t)(gb / T16_RING) & 1u;             // ring phase of this slot's first chunk (gb is 0 or T16_HALF, a multiple of T16_RING)
 #ifdef T16_TRACE
     int trace_n = 0;
 #endif
     // K-chunks are issued in pairs (one fence / elect / two commits per 6 UMMAs): the issuer warp shares its scheduler with two
     // busy worker warps and retires an instruction only every ~24 cycles, so its instruction count per chunk IS its chunk time.
     // The barrier polls of pair kp + 1 are issued before the UMMA block of pair kp.
-    constexpr int NPAIR = T16_NCHUNK / 2, RPAIR = RING / 2, SPAIR = T16_STAGES / 2;
+    constexpr int NPAIR = T16_NCHUNK / 2, RPAIR = T16_RING / 2, SPAIR = T16_STAGES / 2;
     bool rdy_b = t16_mbar_try(smem_u32(&sm.b_full[0]), pb0);
     bool rdy_a0 = t16_mbar_try(smem_u32(&sm.a_full[m][0]), 0u), rdy_a1 = t16_mbar_try(smem_u32(&sm.a_full[m][1]), 0u);
     for (int g0 = gb; g0 < ge; g0 += T16_NCHUNK) {                // one step: stages, ring slots and parities are compile-time
@@ -608,7 +573,7 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
     const int gt = __shfl_sync(0xffffffffu, g_total, 0) / 2;       // chunk pairs (the ranges are multiples of T16_HALF)
     int rp = 0, rphase = 0, kp = 0;
     for (int g = 0; g < gt; ++g) {
-      if (g >= RING / 2) t16_mbar_wait(&sm.b_empty[rp], (uint32_t)(rphase ^ 1));
+      if (g >= T16_RING / 2) t16_mbar_wait(&sm.b_empty[rp], (uint32_t)(rphase ^ 1));
       if (t16_elect_one()) {
         const uint32_t mb = smem_u32(&sm.b_full[rp]);
         asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(mb), "r"(bytes) : "memory");
@@ -617,7 +582,7 @@ __global__ void __launch_bounds__(T16_THREADS, 1) k_rollout_tc16(const __grid_co
                      : "memory");
       }
       __syncwarp();
-      if (++rp == RING / 2) { rp = 0; rphase ^= 1; }
+      if (++rp == T16_RING / 2) { rp = 0; rphase ^= 1; }
       if (++kp == T16_NCHUNK / 2) kp = 0;
     }
   }
@@ -677,6 +642,7 @@ extern "C" int cacto_rollout_tc16(const cacto_sys_params* p, const float* actor_
                                   const int32_t* horizon, int32_t T_max, double* states, double* controls, int32_t* flags,
                                   double* rewards, int64_t B, void* stream) {
   if (!p) return CACTO_E_ARG;
+  if (p->system < CACTO_SINGLE_INTEGRATOR || p->system > CACTO_MANIPULATOR) return CACTO_E_SYSTEM;   // UR5: cacto_rollout_tc
   if (B < 0 || T_max < 0) return CACTO_E_SIZE;
   if (B == 0) return 0;
   if (!actor_params || !w2img || !ics || !horizon || !states || !flags || (T_max > 0 && !controls)) return CACTO_E_ARG;
@@ -689,7 +655,6 @@ extern "C" int cacto_rollout_tc16(const cacto_sys_params* p, const float* actor_
     case CACTO_CAR: return launch_rollout_tc16<CACTO_CAR>(*p, actor_params, img, ics, horizon, T_max, states, controls, flags, rewards, B, st);
     case CACTO_CAR_PARK: return launch_rollout_tc16<CACTO_CAR_PARK>(*p, actor_params, img, ics, horizon, T_max, states, controls, flags, rewards, B, st);
     case CACTO_MANIPULATOR: return launch_rollout_tc16<CACTO_MANIPULATOR>(*p, actor_params, img, ics, horizon, T_max, states, controls, flags, rewards, B, st);
-    case CACTO_UR5: return launch_rollout_tc16<CACTO_UR5>(*p, actor_params, img, ics, horizon, T_max, states, controls, flags, rewards, B, st);
     default: return CACTO_E_SYSTEM;
   }
 }

@@ -3,8 +3,8 @@
 Each op is a thin shim over the extern "C" symbol of the same name in libcacto_b200.so (include/cacto_b200.h): tensors in, raw
 pointers + the current CUDA stream across the C boundary, a non-zero return code raised as RuntimeError.  The Python mirror of
 the reference's modules (environment / NeuralNetwork / RL / replay_buffer / segment_tree / optim / rtg) calls the hot path through
-these ops; what has no op yet (CUDA-IPC peer regions, the generic critic variants, the experimental tf32 / pair-CTA rollout
-engines, the TO backward pass) goes through the same C ABI with ctypes (cacto_b200/_lib.py).
+these ops; what has no op yet (CUDA-IPC peer regions, the generic critic variants, the 3xTF32 rollout engine 'tf32', the TO
+backward pass) goes through the same C ABI with ctypes (cacto_b200/_lib.py).
 
 The shim library is part of the product: importing this module without it raises -- there is no fallback.
 """

@@ -133,7 +133,7 @@ int cacto_rollout_tc(const cacto_sys_params* p, const float* actor_params, const
  *      (a = a_hi + a_lo, w = w_hi + w_lo; a w ~= a_hi w_hi + a_hi w_lo + a_lo w_hi, fp32 accumulation in TMEM: the
  *      accuracy class of 3xTF32 at twice the rate) by persistent CTAs that keep two 128-rollout tiles in flight.
  *      Range limit: hidden activations beyond +-2047 overflow the fp16 high part; such a rollout is flagged failed.
- *      All six systems (UR5 with a 4-slot W2 ring; its fp64 dynamics dominate and cacto_rollout_tc is faster for it).
+ *      The five systems with ns <= 8 and na <= 3; any other, UR5 included, returns CACTO_E_SYSTEM (cacto_rollout_tc runs UR5).
  *      w2img (cacto_actor_tc16_image_bytes() bytes, 128-byte aligned, caller-owned) is the scaled, split, UMMA-laid-out
  *      image of the actor's W2 built by cacto_actor_tc16_prepare; rebuild it whenever the actor changes. */
 int64_t cacto_actor_tc16_image_bytes(void);
@@ -193,15 +193,6 @@ int cacto_actor_grad_generic(const cacto_sys_params* p, const cacto_mlp_desc* d_
                              const cacto_mlp_desc* d_critic, const float* critic_params, const float* state,
                              const float* state_next, const float* Fu, const float* dr_da, float inv_B, float* grad, int64_t B,
                              void* stream);
-
-/* ---- K1 as CTA pairs (tcgen05 cta_group::2): same contract and arithmetic as cacto_rollout_tc16; a cluster of two CTAs steps
- *      256-rollout macro tiles with M = 256 MMAs, each CTA holding half of W2 resident in shared memory (no W2 streaming).
- *      w2img: cacto_actor_tc16p_image_bytes() bytes laid out per CTA rank by cacto_actor_tc16p_prepare. */
-int64_t cacto_actor_tc16p_image_bytes(void);
-int cacto_actor_tc16p_prepare(const float* actor_params, int32_t ns, int32_t na, void* w2img, void* stream);
-int cacto_rollout_tc16p(const cacto_sys_params* p, const float* actor_params, const void* w2img, const double* ics,
-                        const int32_t* horizon, int32_t T_max, double* states, double* controls, int32_t* flags,
-                        double* rewards, int64_t B, void* stream);
 
 /* ---- The actor at any hidden width (conf.NH1 / conf.NH2; NeuralNetwork.py:51-63: ns -> nh1 -> nh2 -> na, LeakyReLU(0.3)),
  *      1 <= nh1, nh2 <= CACTO_ACTOR_MAX_WIDTH, on fp32 CUDA-core kernels that take the widths at run time (csrc/actor_width.cu).

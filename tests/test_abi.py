@@ -118,3 +118,14 @@ def test_product_path_fails_loudly_without_cuda():
     for f in os.listdir(os.path.join(ROOT, 'cacto_b200')):
         if f.endswith('.py'):
             assert 'oracle' not in open(os.path.join(ROOT, 'cacto_b200', f)).read().replace('the oracle', ''), f
+
+
+def test_fp16_rollout_refuses_systems_beyond_its_limits_first():
+    """cacto_rollout_tc16 runs the systems with ns <= 8 and na <= 3; a UR5 parameter block is refused with CACTO_E_SYSTEM
+    before any other argument is looked at, while a supported system still gets to the pointer checks."""
+    import cacto_b200._lib as L
+    from cacto_b200.conf import get_conf
+    null = C.c_void_p(0)
+    for system, code in (('ur5', -2), ('manipulator', -1)):            # CACTO_E_SYSTEM, CACTO_E_ARG
+        P = L.make_sys_params(get_conf(system))
+        assert L.lib.cacto_rollout_tc16(C.byref(P), null, null, null, null, 100, null, null, null, null, 64, null) == code, system
