@@ -105,7 +105,11 @@ _SIGNATURES = {
     'cacto_backward_pass_workspace_bytes': (C.c_int64, [C.c_int32, C.c_int32, C.c_int64]),
     'cacto_backward_pass': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_double, C.c_void_p, C.c_void_p,
                                       C.c_void_p]),
-    'cacto_copy2d_to_host': (C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
+    'cacto_ddp_workspace_bytes': (C.c_int64, [C.c_int32, C.c_int32, C.c_int64, C.c_int32]),
+    'cacto_ddp_init': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64] + [C.c_void_p] * 5),
+    'cacto_ddp_iterate': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_void_p, C.c_void_p, C.c_int64, C.c_int32, C.c_double] +
+                          [C.c_void_p] * 5),
+    'cacto_copy2d_to_host':(C.c_int, [C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_void_p]),
     'cacto_copy3d_to_host': (C.c_int, [C.c_void_p, C.c_int64, C.c_int64, C.c_void_p, C.c_int64, C.c_int64, C.c_int64, C.c_int64, C.c_int64,
                                        C.c_void_p]),
     'cacto_narrow_f64_to_f32': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p]),

@@ -154,6 +154,45 @@ int64_t cacto_backward_pass_workspace_bytes(int32_t nx, int32_t na, int64_t n_kn
 int cacto_backward_pass(const cacto_sys_params* p, const int64_t* offsets, int32_t E, const double* states,
                         const double* controls, int64_t n_knots, double mu, void* workspace, double* V_x, void* stream);
 
+/* ---- K7: the TO solve (TO.py:35-100 solves it with ipopt on the host) as batched iLQR on the GPU, an opt-in alternative.
+ *      Problem, per trajectory e with knots offsets[e] .. offsets[e+1]-1 (T_e = knots - 1 controls): from x_0 = states[offsets[e]]
+ *      (kept fixed) minimise over u_0 .. u_{T-1}
+ *          J = sum_{k<T} c_run(x_k, u_k) + c_term(x_T),   x_{k+1} = Env.simulate(x_k, u_k) in fp64,
+ *      c = -reward (running / terminal weights) with the bounded control cost a^2 + w_b (a/u_max)^10 for every system (UR5
+ *      included): the cost K6 differentiates, with the sign flipped.  No hard bounds (the reference's TO has only the penalty).
+ *      One iteration per trajectory still running: per-knot derivatives at the iterate (K6's knot code); a warp-per-trajectory
+ *      backward recursion with a Cholesky factor of Q_uu + mu I (not positive definite at some knot: the pass fails, mu grows)
+ *      giving k_t = -Quu~^-1 Q_u, K_t = -Quu~^-1 Q_ux and the expected change dV(a) = a dV1 + a^2/2 dV2 (dV1 = sum k'Q_u,
+ *      dV2 = sum k'Q_uu k); CACTO_DDP_N_ALPHA closed-loop probes u = u_bar + a k + K (x - x_bar), a = 2^-j, cost only;
+ *      then the largest a with (J - J(a)) >= CACTO_DDP_C1 (-dV(a)) is re-rolled with the same arithmetic and committed.
+ *      mu: / CACTO_DDP_MU_FACTOR (floor CACTO_DDP_MU_MIN) on success, * CACTO_DDP_MU_FACTOR on failure.
+ *      Status: CONVERGED when |dV(1)| < tol |J| (no step) or an accepted step improved J by < tol |J|; FAILED when mu exceeds
+ *      CACTO_DDP_MU_MAX or the warm start's cost is not finite (the iterate is the last accepted one: the best).
+ *      states[n_knots][nx] (no time column) and controls[n_knots][na] hold the iterate in place (the control row of a
+ *      trajectory's last knot is not used); cost[E] fp64, status[E] int32, iters[E] int32.
+ *      workspace: cacto_ddp_workspace_bytes(nx, na, n_knots, E) bytes, 8-byte aligned, caller-owned: per knot K6's block
+ *      [l_x | l_xx | A | B | l_u | l_uu] followed by [k | K], then per trajectory CACTO_DDP_TRAJ_DOUBLES doubles
+ *      [mu, dV1, dV2, backward ok, probe costs[CACTO_DDP_N_ALPHA], accepted alpha index of iterations 1..CACTO_DDP_HISTORY
+ *      (j >= 0; CACTO_DDP_H_* otherwise)].
+ *      cacto_ddp_init: re-simulates every iterate from x_0 (states written from knot 1 on), sets cost, status, iters = 0, mu.
+ *      cacto_ddp_iterate: n_iter iterations, enqueued without host synchronisation; finished trajectories are skipped. */
+#define CACTO_DDP_N_ALPHA 8
+#define CACTO_DDP_C1 1e-4
+#define CACTO_DDP_MU_INIT 1e-6
+#define CACTO_DDP_MU_MIN 1e-9
+#define CACTO_DDP_MU_MAX 1e10
+#define CACTO_DDP_MU_FACTOR 10.0
+#define CACTO_DDP_HISTORY 8
+#define CACTO_DDP_TRAJ_DOUBLES 24
+enum { CACTO_DDP_RUNNING = 0, CACTO_DDP_CONVERGED = 1, CACTO_DDP_FAILED = 2 };
+enum { CACTO_DDP_H_BACKWARD_FAILED = -1, CACTO_DDP_H_NO_STEP = -2, CACTO_DDP_H_CONVERGED = -3, CACTO_DDP_H_NOT_RUN = -4 };
+int64_t cacto_ddp_workspace_bytes(int32_t nx, int32_t na, int64_t n_knots, int32_t E);
+int cacto_ddp_init(const cacto_sys_params* p, const int64_t* offsets, int32_t E, double* states, const double* controls,
+                   int64_t n_knots, void* workspace, double* cost, int32_t* status, int32_t* iters, void* stream);
+int cacto_ddp_iterate(const cacto_sys_params* p, const int64_t* offsets, int32_t E, double* states, double* controls,
+                      int64_t n_knots, int32_t n_iter, double tol, void* workspace, double* cost, int32_t* status, int32_t* iters,
+                      void* stream);
+
 /* ---- plumbing for the host feeder (main.py:216-233 hands warm-starts to the TO pool): strided device-to-host copy of a
  *      column block, rows x width_bytes, on the copy engine. */
 int cacto_copy2d_to_host(void* dst_host, int64_t dst_pitch, const void* src_dev, int64_t src_pitch, int64_t width_bytes,
