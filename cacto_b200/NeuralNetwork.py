@@ -9,6 +9,10 @@ reference uses: ``trainable_variables`` / ``variables``, ``get_weights`` / ``set
   NN.compute_critic_grad  -> cacto_critic_grad                            (NeuralNetwork.py:150-178)
   NN.compute_actor_grad   -> cacto_actor_grad                             (NeuralNetwork.py:180-232)
 
+``NN(..., deterministic=True)`` runs the 'sine' critic and actor gradients through the ``*_grad_det`` / ``*_grad_tc_det`` entry points:
+the same kernels of both update engines with every cross-CTA and cross-warp sum taken in a fixed order (include/cacto_b200.h), so
+that an update repeated on the same inputs gives the same bits.
+
 An actor whose hidden widths (conf.NH1, conf.NH2) are not 256 is an ``'actor_width'`` network: the same Keras layout and layer
 names, no transposed copy, run by the width-generic kernels of csrc/actor_width.cu (cacto_rollout_width / cacto_actor_forward_width /
 cacto_actor_grad_width) with the widths passed at run time.
@@ -156,10 +160,17 @@ def _glorot(rng, i, o):
 class NN:
     """NeuralNetwork.py:10-232."""
 
-    def __init__(self, env, conf, w_S=0, seed=None):
+    def __init__(self, env, conf, w_S=0, seed=None, deterministic=False):
+        """``deterministic``: bit-reproducible gradients (fixed-order sums instead of fp32 atomics) for the 'sine' critic and its
+        actor.  For a fixed GPU model, build, system, batch size and world size the same inputs then give the same bits in every
+        gradient, weight, Adam moment, rtg, V, V_target and ``last_critic_loss``.  The generic critic variants have no such path."""
         self.env = env
         self.conf = conf
         self.w_S = w_S
+        self.deterministic = bool(deterministic)
+        if self.deterministic and getattr(conf, 'critic_type', 'sine') != 'sine':
+            raise ValueError(f"deterministic=True needs critic_type 'sine' (got {conf.critic_type!r}): the generic critic kernels sum "
+                             'their gradients with one atomic per weight and sample')
         self._rng = np.random.default_rng(seed)
         self._p = env._p
         self._pt = env._pt
@@ -276,6 +287,21 @@ class NN:
             raise ValueError('unknown update engine %r' % (eng,))
         return eng == 'tc' or (eng == 'auto' and B >= self.TC_MIN_BATCH)
 
+    # partials workspace of the deterministic gradients: one per network and engine (the pipelined update runs the critic and actor
+    # gradients concurrently), sized for the batch (ops.det_partials_floats stops growing above CACTO_DET_MAX_SLICES tiles).  A
+    # workspace that is outgrown is kept, not freed: a CUDA graph captured with it (RL.UpdateGraph) still writes to it on replay.
+    DET_CRITIC, DET_ACTOR, DET_ACTOR_WIDTH, DET_CRITIC_TC, DET_ACTOR_TC = 0, 1, 2, 3, 4
+
+    def _det_partials(self, net, B, nh1=0, nh2=0):
+        need = int(ops.det_partials_floats(net, B, self.conf.nb_state, self.conf.nb_action, nh1, nh2))
+        cache = self.__dict__.setdefault('_det_ws', {})
+        ws = cache.get(net)
+        if ws is None or ws.numel() < need:
+            if ws is not None:
+                self.__dict__.setdefault('_det_ws_outgrown', []).append(ws)
+            ws = cache[net] = torch.empty(need, dtype=torch.float32, device=_device())
+        return ws
+
     def _tc_workspace(self, B):
         need = int(ops.update_tc_workspace_bytes(B, self.conf.nb_state, self.conf.nb_action))
         ws = getattr(self, '_tc_ws', None)
@@ -285,6 +311,10 @@ class NN:
         return ws
 
     def launch_critic_grad(self, cm, tc, s, sn, pr, dv, d, w, inv_B, rtg, V, Vt, B):
+        if cm.kind == 'critic_sine' and self._use_tc(B) and self.deterministic:
+            ops.critic_grad_tc_det(self._pt, cm.params, tc.params, float(self.w_S), int(bool(self.conf.MC)), s, sn, pr, dv, d, w, inv_B, cm.grad, rtg, V, Vt,
+                                   self.last_critic_loss, self._tc_workspace(B), self._det_partials(self.DET_CRITIC_TC, B))
+            return
         if cm.kind == 'critic_sine' and self._use_tc(B):
             ws = self._tc_workspace(B)
             ops.critic_grad_tc(self._pt, cm.params, tc.params, float(self.w_S), int(bool(self.conf.MC)), s, sn, pr, dv, d, w, inv_B, cm.grad, rtg, V, Vt,
@@ -294,13 +324,24 @@ class NN:
             check(lib.cacto_critic_grad_generic(self._p, _lib.C.byref(cm.desc), ptr(cm.params), ptr(tc.params), float(self.w_S),
                                                 int(bool(self.conf.MC)), ptr(s), ptr(sn), ptr(pr), ptr(dv), ptr(d), ptr(w), inv_B, ptr(cm.grad),
                                                 ptr(rtg), ptr(V), ptr(Vt), ptr(self.last_critic_loss), B, stream_ptr()), 'critic_grad_generic')
+        elif self.deterministic:
+            ops.critic_grad_det(self._pt, cm.params, cm.params_T, tc.params, float(self.w_S), int(bool(self.conf.MC)), s, sn, pr, dv, d, w, inv_B, cm.grad, rtg,
+                                V, Vt, self.last_critic_loss, self._det_partials(self.DET_CRITIC, B))
         else:
             ops.critic_grad(self._pt, cm.params, cm.params_T, tc.params, float(self.w_S), int(bool(self.conf.MC)), s, sn, pr, dv, d, w, inv_B, cm.grad, rtg, V, Vt,
                             self.last_critic_loss)
 
     def launch_actor_grad(self, am, cm, s, term, inv_B, actions, B):
+        if am.kind == 'actor_width' and cm.kind == 'critic_sine' and self.deterministic:
+            ops.actor_grad_width_det(self._pt, am.params, am.dims[1], am.dims[2], cm.params, cm.params_T, s, term, inv_B, am.grad, actions,
+                                     self._det_partials(self.DET_ACTOR_WIDTH, B, am.dims[1], am.dims[2]))
+            return
         if am.kind == 'actor_width' and cm.kind == 'critic_sine':      # whatever the batch size: the tcgen05 engine is 256-wide only
             ops.actor_grad_width(self._pt, am.params, am.dims[1], am.dims[2], cm.params, cm.params_T, s, term, inv_B, am.grad, actions)
+            return
+        if cm.kind == 'critic_sine' and self._use_tc(B) and self.deterministic:
+            ops.actor_grad_tc_det(self._pt, am.params, cm.params, s, term, inv_B, am.grad, actions, self._tc_workspace(B),
+                                  self._det_partials(self.DET_ACTOR_TC, B))
             return
         if cm.kind == 'critic_sine' and self._use_tc(B):
             ws = self._tc_workspace(B)
@@ -325,6 +366,9 @@ class NN:
                 actions.copy_(act)
             check(lib.cacto_actor_grad_generic(self._p, _lib.C.byref(am.desc), ptr(am.params), _lib.C.byref(cm.desc), ptr(cm.params), ptr(s),
                                                ptr(s_next), ptr(Fu), ptr(dr_da), inv_B, ptr(am.grad), B, stream_ptr()), 'actor_grad_generic')
+        elif self.deterministic:
+            ops.actor_grad_det(self._pt, am.params, am.params_T, cm.params, cm.params_T, s, term, inv_B, am.grad, actions,
+                               self._det_partials(self.DET_ACTOR, B))
         else:
             ops.actor_grad(self._pt, am.params, am.params_T, cm.params, cm.params_T, s, term, inv_B, am.grad, actions)
 

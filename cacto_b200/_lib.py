@@ -141,6 +141,16 @@ _SIGNATURES = {
     'cacto_critic_grad_tc': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int] + [C.c_void_p] * 6 + [C.c_float] + [C.c_void_p] * 5 +
                              [C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
     'cacto_actor_grad_tc': (C.c_int, [C.c_void_p] * 5 + [C.c_float, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    'cacto_det_partials_floats': (C.c_int64, [C.c_int32, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
+    'cacto_critic_grad_det': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int] + [C.c_void_p] * 6 +
+                              [C.c_float] + [C.c_void_p] * 5 + [C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    'cacto_actor_grad_det': (C.c_int, [C.c_void_p] * 7 + [C.c_float, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    'cacto_actor_grad_width_det': (C.c_int, [C.c_void_p, C.c_void_p, C.c_int32, C.c_int32] + [C.c_void_p] * 4 + [C.c_float, C.c_void_p, C.c_void_p,
+                                                                                                            C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    'cacto_critic_grad_tc_det': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_float, C.c_int] + [C.c_void_p] * 6 + [C.c_float] +
+                                 [C.c_void_p] * 5 + [C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p]),
+    'cacto_actor_grad_tc_det': (C.c_int, [C.c_void_p] * 5 + [C.c_float, C.c_void_p, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64, C.c_void_p, C.c_int64,
+                                          C.c_void_p]),
     'cacto_adam_schedule': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),
     'cacto_adam_schedule2': (C.c_int, [C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float, C.c_float, C.c_void_p,
                                       C.c_void_p, C.c_void_p, C.c_void_p, C.c_int32, C.c_float, C.c_float, C.c_void_p, C.c_void_p, C.c_void_p]),

@@ -12,6 +12,7 @@
 //              output unit, lanes stride the weight row (coalesced), per-sample partial sums meet in a shuffle butterfly.
 //   wouter     dW[K x N] += A^T E over the CTA's tile of samples: ONE fp32 atomic per weight and tile (not per sample).
 #include "common.cuh"
+#include "det.cuh"
 #include "mlp.cuh"
 #include "systems.cuh"
 
@@ -110,6 +111,7 @@ __device__ __forceinline__ void wgemm_nt(const float* E, int lde, int K, const f
 }
 
 // dW[k][n] += sum_{s < rows} A[s][k] E[s][n], k < K, n < N (dW row stride N).  A: [S][lda], lda % 4 == 0, lda >= round4(K).
+template <bool DET = false>
 __device__ __forceinline__ void wouter(const float* A, int lda, const float* E, int lde, int K, int N, float* __restrict__ dW, int rows) {
   const int kq = (K + 3) >> 2;
   for (int t = threadIdx.x; t < kq * N; t += AW_NT) {
@@ -125,7 +127,7 @@ __device__ __forceinline__ void wouter(const float* A, int lda, const float* E, 
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i)
-      if (k0 + i < K) atomicAdd(dW + (size_t)(k0 + i) * N + n, acc[i]);
+      if (k0 + i < K) grad_add<DET>(dW + (size_t)(k0 + i) * N + n, acc[i]);
   }
 }
 
@@ -254,7 +256,8 @@ __host__ __device__ __forceinline__ size_t ag_smem_bytes(int S, int h1, int h2) 
   return 4u * (size_t)S * (3 * AW_NSP + 3 * AW_NAP + AW_FUP + AW_CW + 2 * CR_H4 + round4(h1) + max(round4(h1), round4(h2)) + round4(h2));
 }
 
-template <int SYS, int S>
+// DET: grad is the partials workspace (det.cuh); the CTA adds into its slice
+template <int SYS, int S, bool DET = false>
 __global__ void __launch_bounds__(AW_NT) k_actor_grad_width(const __grid_constant__ cacto_sys_params P, const float* __restrict__ aw, int h1, int h2,
                                                             const float* __restrict__ cw, const float* __restrict__ cwT,
                                                             const float* __restrict__ state, const double* __restrict__ term, float inv_B,
@@ -278,6 +281,7 @@ __global__ void __launch_bounds__(AW_NT) k_actor_grad_width(const __grid_constan
   float* E = H2 + S * max(ld1, ld2);              // [S][ld2] dL/dz2
   const ActorLayout LA(NS, NA, h1, h2);
   const CriticLayout LC(NS);
+  if constexpr (DET) grad += (size_t)blockIdx.x * det_stride(LA.total);
   const int tid = threadIdx.x;
   const int64_t row0 = (int64_t)blockIdx.x * S;
   const int rows = (int)min((int64_t)S, B - row0);
@@ -385,12 +389,12 @@ __global__ void __launch_bounds__(AW_NT) k_actor_grad_width(const __grid_constan
     const int k = i / NA, j = i - k * NA;
     float acc = 0.f;
     for (int s = 0; s < rows; ++s) acc = fmaf(H2[s * ld2 + k], D3[s * AW_NAP + j], acc);
-    atomicAdd(grad + LA.W3 + i, acc);
+    grad_add<DET>(grad + LA.W3 + i, acc);
   }
   if (tid < NA) {
     float acc = 0.f;
     for (int s = 0; s < rows; ++s) acc += D3[s * AW_NAP + tid];
-    atomicAdd(grad + LA.b3 + tid, acc);
+    grad_add<DET>(grad + LA.b3 + tid, acc);
   }
   for (int i = tid; i < S * h2; i += AW_NT) {                  // e2 = (d3 W3^T) * lrelu'(z2)
     const int s = i / h2, n = i - s * h2;
@@ -400,14 +404,14 @@ __global__ void __launch_bounds__(AW_NT) k_actor_grad_width(const __grid_constan
     E[s * ld2 + n] = acc * (H2[s * ld2 + n] > 0.f ? 1.f : LEAKY_ALPHA);
   }
   __syncthreads();
-  wouter(H1, ld1, E, ld2, h1, h2, grad + LA.W2, rows);
-  tile_colsum<AW_NT>(E, ld2, h2, rows, grad + LA.b2);
+  wouter<DET>(H1, ld1, E, ld2, h1, h2, grad + LA.W2, rows);
+  tile_colsum<AW_NT, DET>(E, ld2, h2, rows, grad + LA.b2);
   // e1 = (e2 W2^T) * lrelu'(z1), re-strided to ld1, into the buffer of H2 (dead once e2 is formed; sized for either stride)
   float* E1 = H2;
   wgemm_nt<S>(E, ld2, h2, aw + LA.W2, h2, h1, [&](int s, int i, float v) { E1[s * ld1 + i] = v * (H1[s * ld1 + i] > 0.f ? 1.f : LEAKY_ALPHA); });
   __syncthreads();
-  wouter(XN, AW_NSP, E1, ld1, NS, h1, grad + LA.W1, rows);
-  tile_colsum<AW_NT>(E1, ld1, h1, rows, grad + LA.b1);
+  wouter<DET>(XN, AW_NSP, E1, ld1, NS, h1, grad + LA.W1, rows);
+  tile_colsum<AW_NT, DET>(E1, ld1, h1, rows, grad + LA.b1);
 }
 
 template <typename K>
@@ -447,12 +451,36 @@ static int launch_actor_grad_width_s(const cacto_sys_params& P, const float* aw,
   return 0;
 }
 
-// 4-sample tiles while they fill at most one wave of the 148 SMs (latency of the reference's batch sizes), 16-sample tiles beyond
 template <int SYS>
 static int launch_actor_grad_width(const cacto_sys_params& P, const float* aw, int h1, int h2, const float* cw, const float* cwT, const float* state,
                                    const double* term, float inv_B, float* grad, float* actions, int64_t B, cudaStream_t st) {
-  if (B <= 4 * 148) return launch_actor_grad_width_s<SYS, 4>(P, aw, h1, h2, cw, cwT, state, term, inv_B, grad, actions, B, st);
+  if (actor_width_tile(B) == 4) return launch_actor_grad_width_s<SYS, 4>(P, aw, h1, h2, cw, cwT, state, term, inv_B, grad, actions, B, st);
   return launch_actor_grad_width_s<SYS, 16>(P, aw, h1, h2, cw, cwT, state, term, inv_B, grad, actions, B, st);
+}
+
+// deterministic variant: DET = true in waves of at most CACTO_DET_MAX_SLICES CTAs, then the fixed-order reduce (det.cuh)
+template <int SYS, int S>
+static int actor_grad_width_det_s(const cacto_sys_params& P, const float* aw, int h1, int h2, const float* cw, const float* cwT, const float* state,
+                                  const double* term, float inv_B, float* grad, float* actions, int64_t B, float* part, cudaStream_t st) {
+  auto k = k_actor_grad_width<SYS, S, true>;
+  const size_t sm = ag_smem_bytes(S, h1, h2);
+  if (int e = aw_smem_attr(k, sm)) return e;
+  const int64_t n = ActorLayout(P.ns, P.na, h1, h2).total, tiles = (B + S - 1) / S, slices = det_slices(tiles), ns = P.ns, na = P.na;
+  if (cudaError_t e = cudaMemsetAsync(part, 0, (size_t)(slices * det_stride(n)) * sizeof(float), st)) return (int)e;
+  for (int64_t t0 = 0; t0 < tiles; t0 += slices) {
+    const int64_t r0 = t0 * S, rows = B - r0 < slices * S ? B - r0 : slices * S;
+    if (cudaError_t le = launch_pdl(k, (unsigned)((rows + S - 1) / S), AW_NT, sm, st, P, aw, h1, h2, cw, cwT, state + r0 * ns, term + r0, inv_B, part,
+                                    actions ? actions + r0 * na : nullptr, rows))
+      return (int)le;
+    CACTO_LAUNCH_CHECK();
+  }
+  return det_reduce(part, slices, n, grad, nullptr, st);
+}
+template <int SYS>
+static int actor_grad_width_det(const cacto_sys_params& P, const float* aw, int h1, int h2, const float* cw, const float* cwT, const float* state,
+                                const double* term, float inv_B, float* grad, float* actions, int64_t B, float* part, cudaStream_t st) {
+  if (actor_width_tile(B) == 4) return actor_grad_width_det_s<SYS, 4>(P, aw, h1, h2, cw, cwT, state, term, inv_B, grad, actions, B, part, st);
+  return actor_grad_width_det_s<SYS, 16>(P, aw, h1, h2, cw, cwT, state, term, inv_B, grad, actions, B, part, st);
 }
 
 static bool aw_width_ok(int32_t h) { return h >= 1 && h <= CACTO_ACTOR_MAX_WIDTH; }
@@ -515,4 +543,19 @@ extern "C" int cacto_actor_grad_width(const cacto_sys_params* p, const float* ac
   if (B == 0) return 0;
   cudaStream_t st = (cudaStream_t)stream;
   AW_DISPATCH(launch_actor_grad_width, *p, actor_params, nh1, nh2, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, st)
+}
+
+extern "C" int cacto_actor_grad_width_det(const cacto_sys_params* p, const float* actor_params, int32_t nh1, int32_t nh2, const float* critic_params,
+                                          const float* critic_params_T, const float* state, const double* term, float inv_B, float* grad,
+                                          float* actions, int64_t B, float* partials, int64_t partials_floats, void* stream) {
+  if (!p) return CACTO_E_ARG;
+  if (!aw_width_ok(nh1) || !aw_width_ok(nh2) || B < 0) return CACTO_E_SIZE;
+  if (!actor_params || !critic_params || !critic_params_T || !state || !term || !grad || !partials) return CACTO_E_ARG;
+  if (!aw_aligned16(actor_params) || !aw_aligned16(critic_params) || !aw_aligned16(critic_params_T) || !aw_aligned16(grad) || !aw_aligned16(partials))
+    return CACTO_E_ALIGN;
+  if (B == 0) return 0;
+  const int64_t need = cacto_det_partials_floats(CACTO_DET_ACTOR_WIDTH, B, p->ns, p->na, nh1, nh2);
+  if (need < 0 || partials_floats < need) return CACTO_E_SIZE;
+  cudaStream_t st = (cudaStream_t)stream;
+  AW_DISPATCH(actor_grad_width_det, *p, actor_params, nh1, nh2, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, partials, st)
 }

@@ -313,9 +313,29 @@ __device__ __forceinline__ void tile_gemm_small(const float* __restrict__ A, int
   }
 }
 
-// dW[k][n] += scale-free sum_s A1[s][k] E1[s][n] (+ A2[s][k] E2[s][n]); K x N outputs, atomics to global.
+// Adding a CTA's contribution into a gradient block.  DET = false: fp32 atomics into the shared accumulator (the order in which the
+// CTAs land decides the low bits).  DET = true: the block is the CTA's own partials slice (csrc/det.cuh), which no other CTA
+// touches, and each element is written by one thread of the CTA -- a plain read-modify-write in program order.
+template <bool DET>
+__device__ __forceinline__ void grad_add(float* p, float v) {
+  if constexpr (DET) *p += v;
+  else atomicAdd(p, v);
+}
+template <bool DET>
+__device__ __forceinline__ void grad_add4(float* p, const float4& v) {
+  if constexpr (DET) {
+    float4 g = *reinterpret_cast<float4*>(p);
+    g.x += v.x; g.y += v.y; g.z += v.z; g.w += v.w;
+    *reinterpret_cast<float4*>(p) = g;
+  } else {
+    // one 16-byte vector reduction (red.global.add.v4.f32, sm_90+) instead of four scalar ones
+    atomicAdd(reinterpret_cast<float4*>(p), v);
+  }
+}
+
+// dW[k][n] += scale-free sum_s A1[s][k] E1[s][n] (+ A2[s][k] E2[s][n]); K x N outputs, atomics to global (grad_add).
 // A*: shared [S][lda*] (k contiguous), E*: shared [S][lde*].  Rows k >= K are skipped.  KT = 4.  dW must be 16-byte aligned.
-template <int S, int N, int NT>
+template <int S, int N, int NT, bool DET = false>
 __device__ __forceinline__ void tile_outer2(const float* __restrict__ A1, int lda1, const float* __restrict__ E1, int lde1,
                                             const float* __restrict__ A2, int lda2, const float* __restrict__ E2, int lde2, int K,
                                             float* __restrict__ dW, int rows_valid) {
@@ -347,22 +367,19 @@ __device__ __forceinline__ void tile_outer2(const float* __restrict__ A1, int ld
     }
 #pragma unroll
     for (int i = 0; i < 4; ++i) {
-      if (k0 + i < K) {
-        // one 16-byte vector reduction (red.global.add.v4.f32, sm_90+) instead of four scalar ones: the weight matrices
-        // start at multiples of 4 floats inside the 16-byte-aligned gradient block, N % 4 == 0
-        atomicAdd(reinterpret_cast<float4*>(dW + (size_t)(k0 + i) * N + 4 * cg), acc[i]);
-      }
+      // 16-byte accesses: the weight matrices start at multiples of 4 floats inside the 16-byte-aligned gradient block, N % 4 == 0
+      if (k0 + i < K) grad_add4<DET>(dW + (size_t)(k0 + i) * N + 4 * cg, acc[i]);
     }
   }
 }
 
 // db[n] += sum_s E[s][n]
-template <int NT>
+template <int NT, bool DET = false>
 __device__ __forceinline__ void tile_colsum(const float* __restrict__ E, int lde, int N, int rows_valid, float* __restrict__ db) {
   for (int n = threadIdx.x; n < N; n += NT) {
     float acc = 0.f;
     for (int s = 0; s < rows_valid; ++s) acc += E[s * lde + n];
-    atomicAdd(db + n, acc);
+    grad_add<DET>(db + n, acc);
   }
 }
 

@@ -321,7 +321,9 @@ __device__ __forceinline__ float acc_absmax(const Epi& e) {
   }
   return m;
 }
-// column sums over the 32 rows of a warp for 16 columns (butterfly: 16 shuffles), added into colsum[c0 .. c0 + 15]
+// column sums over the 32 rows of a warp for 16 columns (butterfly: 16 shuffles), added into colsum[c0 .. c0 + 15].  DET: colsum
+// belongs to this warp alone (a per-quadrant copy, update_tc.cu), so each lane adds its column with a plain read-modify-write.
+template <bool DET = false>
 __device__ __forceinline__ void warp_colsum16(float* colsum, int c0, const float* v, int lane) {
   float a[8];
   {
@@ -354,7 +356,11 @@ __device__ __forceinline__ void warp_colsum16(float* colsum, int c0, const float
   float d = (up ? c[1] : c[0]) + __shfl_xor_sync(0xffffffffu, up ? c[0] : c[1], 2);
   d += __shfl_xor_sync(0xffffffffu, d, 1);
   // lane holds column 8 [lane & 16] + 4 [lane & 8] + 2 [lane & 4] + [lane & 2]
-  if ((lane & 1) == 0) atomicAdd(&colsum[c0 + ((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1)], d);
+  if ((lane & 1) == 0) {
+    float* p = &colsum[c0 + ((lane >> 4) & 1) * 8 + ((lane >> 3) & 1) * 4 + ((lane >> 2) & 1) * 2 + ((lane >> 1) & 1)];
+    if constexpr (DET) *p += d;
+    else atomicAdd(p, d);
+  }
 }
 __device__ __forceinline__ void amax_update(uint32_t* slot, float m, int lane) {      // slot = max over the tensor of |x| (bit pattern)
   uint32_t b = __float_as_uint(m) & 0x7fffffffu;

@@ -205,6 +205,86 @@ void actor_grad(const Tensor& p, const Tensor& actor, const Tensor& actor_T, con
                       (const float*)dev(critic_T, F32, "critic_T"), (const float*)dev(state, F32, "state"), (const double*)dev(term, F64, "term"), (float)inv_B,
                       (float*)dev(grad, F32, "grad"), (float*)opt(actions, F32, "actions"), B, stream()), "actor_grad");
 }
+// ---- deterministic gradients (fixed-order sums through a partials workspace of det_partials_floats elements)
+int64_t det_partials_floats(int64_t net, int64_t B, int64_t ns, int64_t na, int64_t nh1, int64_t nh2) {
+  return cacto_det_partials_floats((int32_t)net, B, (int32_t)ns, (int32_t)na, (int32_t)nh1, (int32_t)nh2);
+}
+int64_t det_need(int32_t net, int64_t B, const cacto_sys_params* P_, int64_t nh1, int64_t nh2, const Tensor& partials) {
+  const int64_t n = cacto_det_partials_floats(net, B, P_->ns, P_->na, (int32_t)nh1, (int32_t)nh2);
+  TORCH_CHECK(n >= 0, "cacto: no deterministic workspace size for these arguments");
+  need_at_least(partials, n, "partials");
+  return partials.numel();
+}
+void critic_grad_det(const Tensor& p, const Tensor& critic, const Tensor& critic_T, const Tensor& target, double w_S, int64_t mc, const Tensor& state,
+                     const optional<Tensor>& state_next, const Tensor& prtg, const optional<Tensor>& dVdx, const optional<Tensor>& done, const Tensor& weights,
+                     double inv_B, Tensor grad, Tensor rtg, Tensor V, Tensor Vt, const optional<Tensor>& loss, Tensor partials) {
+  const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
+  const int64_t B = rows_of(state, P_->ns, "state"), nc = cacto_critic_param_count(P_->ns);
+  need(critic, nc, "critic"); need(target, nc, "target"); need(grad, nc, "grad");
+  need(state_next, B * P_->ns, "state_next"); need(prtg, B, "partial_rtg"); need(dVdx, B * P_->ns, "dVdx"); need(done, B, "done"); need(weights, B, "weights");
+  need(rtg, B, "rtg"); need(V, B, "V"); need(Vt, B, "V_target"); need(loss, 1, "loss");
+  need(critic_T, nc, "critic_T");
+  const int64_t np = det_need(CACTO_DET_CRITIC, B, P_, 0, 0, partials);
+  ok(cacto_critic_grad_det(P_, (const float*)dev(critic, F32, "critic"), (const float*)dev(critic_T, F32, "critic_T"), (const float*)dev(target, F32, "target"),
+                           (float)w_S, (int)mc, (const float*)dev(state, F32, "state"), (const float*)opt(state_next, F32, "state_next"),
+                           (const float*)dev(prtg, F32, "partial_rtg"), (const float*)opt(dVdx, F32, "dVdx"), (const float*)opt(done, F32, "done"),
+                           (const float*)dev(weights, F32, "weights"), (float)inv_B, (float*)dev(grad, F32, "grad"), (float*)dev(rtg, F32, "rtg"),
+                           (float*)dev(V, F32, "V"), (float*)dev(Vt, F32, "V_target"), (float*)opt(loss, F32, "loss"), B,
+                           (float*)dev(partials, F32, "partials"), np, stream()), "critic_grad_det");
+}
+void actor_grad_det(const Tensor& p, const Tensor& actor, const Tensor& actor_T, const Tensor& critic, const Tensor& critic_T, const Tensor& state, const Tensor& term,
+                    double inv_B, Tensor grad, const optional<Tensor>& actions, Tensor partials) {
+  const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
+  const int64_t B = rows_of(state, P_->ns, "state"), nact = cacto_actor_param_count(P_->ns, P_->na);
+  need(actor, nact, "actor"); need(grad, nact, "grad"); need(critic, cacto_critic_param_count(P_->ns), "critic"); need(term, B, "term"); need(actions, B * P_->na, "actions");
+  need(actor_T, nact, "actor_T"); need(critic_T, cacto_critic_param_count(P_->ns), "critic_T");
+  const int64_t np = det_need(CACTO_DET_ACTOR, B, P_, 0, 0, partials);
+  ok(cacto_actor_grad_det(P_, (const float*)dev(actor, F32, "actor"), (const float*)dev(actor_T, F32, "actor_T"), (const float*)dev(critic, F32, "critic"),
+                          (const float*)dev(critic_T, F32, "critic_T"), (const float*)dev(state, F32, "state"), (const double*)dev(term, F64, "term"), (float)inv_B,
+                          (float*)dev(grad, F32, "grad"), (float*)opt(actions, F32, "actions"), B, (float*)dev(partials, F32, "partials"), np, stream()),
+     "actor_grad_det");
+}
+void actor_grad_width_det(const Tensor& p, const Tensor& actor, int64_t nh1, int64_t nh2, const Tensor& critic, const Tensor& critic_T, const Tensor& state,
+                          const Tensor& term, double inv_B, Tensor grad, const optional<Tensor>& actions, Tensor partials) {
+  const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
+  const int64_t B = rows_of(state, P_->ns, "state"), nact = actor_width_count(P_, nh1, nh2), nc = cacto_critic_param_count(P_->ns);
+  need(actor, nact, "actor"); need(grad, nact, "grad"); need(critic, nc, "critic"); need(critic_T, nc, "critic_T"); need(term, B, "term");
+  need(actions, B * P_->na, "actions");
+  const int64_t np = det_need(CACTO_DET_ACTOR_WIDTH, B, P_, nh1, nh2, partials);
+  ok(cacto_actor_grad_width_det(P_, (const float*)dev(actor, F32, "actor"), (int32_t)nh1, (int32_t)nh2, (const float*)dev(critic, F32, "critic"),
+                                (const float*)dev(critic_T, F32, "critic_T"), (const float*)dev(state, F32, "state"), (const double*)dev(term, F64, "term"),
+                                (float)inv_B, (float*)dev(grad, F32, "grad"), (float*)opt(actions, F32, "actions"), B, (float*)dev(partials, F32, "partials"), np,
+                                stream()), "actor_grad_width_det");
+}
+void critic_grad_tc_det(const Tensor& p, const Tensor& critic, const Tensor& target, double w_S, int64_t mc, const Tensor& state,
+                        const optional<Tensor>& state_next, const Tensor& prtg, const optional<Tensor>& dVdx, const optional<Tensor>& done, const Tensor& weights,
+                        double inv_B, Tensor grad, Tensor rtg, Tensor V, Tensor Vt, const optional<Tensor>& loss, Tensor workspace, Tensor partials) {
+  const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
+  const int64_t B = rows_of(state, P_->ns, "state"), nc = cacto_critic_param_count(P_->ns);
+  need(critic, nc, "critic"); need(target, nc, "target"); need(grad, nc, "grad");
+  need(state_next, B * P_->ns, "state_next"); need(prtg, B, "partial_rtg"); need(dVdx, B * P_->ns, "dVdx"); need(done, B, "done"); need(weights, B, "weights");
+  need(rtg, B, "rtg"); need(V, B, "V"); need(Vt, B, "V_target"); need(loss, 1, "loss");
+  need_at_least(workspace, cacto_update_tc_workspace_bytes(B, P_->ns, P_->na), "workspace");
+  const int64_t np = det_need(CACTO_DET_CRITIC_TC, B, P_, 0, 0, partials);
+  ok(cacto_critic_grad_tc_det(P_, (const float*)dev(critic, F32, "critic"), (const float*)dev(target, F32, "target"), (float)w_S, (int)mc,
+                              (const float*)dev(state, F32, "state"), (const float*)opt(state_next, F32, "state_next"), (const float*)dev(prtg, F32, "partial_rtg"),
+                              (const float*)opt(dVdx, F32, "dVdx"), (const float*)opt(done, F32, "done"), (const float*)dev(weights, F32, "weights"), (float)inv_B,
+                              (float*)dev(grad, F32, "grad"), (float*)dev(rtg, F32, "rtg"), (float*)dev(V, F32, "V"), (float*)dev(Vt, F32, "V_target"),
+                              (float*)opt(loss, F32, "loss"), B, dev(workspace, at::kByte, "workspace"), workspace.numel(),
+                              (float*)dev(partials, F32, "partials"), np, stream()), "critic_grad_tc_det");
+}
+void actor_grad_tc_det(const Tensor& p, const Tensor& actor, const Tensor& critic, const Tensor& state, const Tensor& term, double inv_B, Tensor grad,
+                       const optional<Tensor>& actions, Tensor workspace, Tensor partials) {
+  const cacto_sys_params* P_ = sys(p);      // checked before anything else is touched
+  const int64_t B = rows_of(state, P_->ns, "state"), nact = cacto_actor_param_count(P_->ns, P_->na);
+  need(actor, nact, "actor"); need(grad, nact, "grad"); need(critic, cacto_critic_param_count(P_->ns), "critic"); need(term, B, "term"); need(actions, B * P_->na, "actions");
+  need_at_least(workspace, cacto_update_tc_workspace_bytes(B, P_->ns, P_->na), "workspace");
+  const int64_t np = det_need(CACTO_DET_ACTOR_TC, B, P_, 0, 0, partials);
+  ok(cacto_actor_grad_tc_det(P_, (const float*)dev(actor, F32, "actor"), (const float*)dev(critic, F32, "critic"), (const float*)dev(state, F32, "state"),
+                             (const double*)dev(term, F64, "term"), (float)inv_B, (float*)dev(grad, F32, "grad"), (float*)opt(actions, F32, "actions"), B,
+                             dev(workspace, at::kByte, "workspace"), workspace.numel(), (float*)dev(partials, F32, "partials"), np, stream()),
+     "actor_grad_tc_det");
+}
 int64_t update_tc_workspace_bytes(int64_t B, int64_t ns, int64_t na) { return cacto_update_tc_workspace_bytes(B, (int32_t)ns, (int32_t)na); }
 void critic_grad_tc(const Tensor& p, const Tensor& critic, const Tensor& target, double w_S, int64_t mc, const Tensor& state, const optional<Tensor>& state_next,
                     const Tensor& prtg, const optional<Tensor>& dVdx, const optional<Tensor>& done, const Tensor& weights, double inv_B, Tensor grad, Tensor rtg, Tensor V,
@@ -329,6 +409,19 @@ TORCH_LIBRARY(cacto, m) {
         "Tensor weights, float inv_B, Tensor(a!) grad, Tensor(b!) rtg, Tensor(c!) V, Tensor(d!) Vt, Tensor(e!)? loss, Tensor(f!) workspace) -> ()", critic_grad_tc);
   m.def("actor_grad_tc(Tensor p, Tensor actor, Tensor critic, Tensor state, Tensor term, float inv_B, Tensor(a!) grad, Tensor(b!)? actions, Tensor(c!) workspace) -> ()",
         actor_grad_tc);
+  m.def("det_partials_floats(int net, int B, int ns, int na, int nh1, int nh2) -> int", det_partials_floats);
+  m.def("critic_grad_det(Tensor p, Tensor critic, Tensor critic_T, Tensor target, float w_S, int mc, Tensor state, Tensor? state_next, Tensor prtg, "
+        "Tensor? dVdx, Tensor? done, Tensor weights, float inv_B, Tensor(a!) grad, Tensor(b!) rtg, Tensor(c!) V, Tensor(d!) Vt, Tensor(e!)? loss, "
+        "Tensor(f!) partials) -> ()", critic_grad_det);
+  m.def("actor_grad_det(Tensor p, Tensor actor, Tensor actor_T, Tensor critic, Tensor critic_T, Tensor state, Tensor term, float inv_B, Tensor(a!) grad, "
+        "Tensor(b!)? actions, Tensor(c!) partials) -> ()", actor_grad_det);
+  m.def("actor_grad_width_det(Tensor p, Tensor actor, int nh1, int nh2, Tensor critic, Tensor critic_T, Tensor state, Tensor term, float inv_B, "
+        "Tensor(a!) grad, Tensor(b!)? actions, Tensor(c!) partials) -> ()", actor_grad_width_det);
+  m.def("critic_grad_tc_det(Tensor p, Tensor critic, Tensor target, float w_S, int mc, Tensor state, Tensor? state_next, Tensor prtg, Tensor? dVdx, "
+        "Tensor? done, Tensor weights, float inv_B, Tensor(a!) grad, Tensor(b!) rtg, Tensor(c!) V, Tensor(d!) Vt, Tensor(e!)? loss, Tensor(f!) workspace, "
+        "Tensor(g!) partials) -> ()", critic_grad_tc_det);
+  m.def("actor_grad_tc_det(Tensor p, Tensor actor, Tensor critic, Tensor state, Tensor term, float inv_B, Tensor(a!) grad, Tensor(b!)? actions, "
+        "Tensor(c!) workspace, Tensor(d!) partials) -> ()", actor_grad_tc_det);
   m.def("adam_schedule(Tensor(a!) step, Tensor boundaries, Tensor values, int nb, float beta1, float beta2, Tensor(b!) alpha, Tensor(c!)? zero) -> ()", adam_schedule);
   m.def("adam_schedule2(Tensor(a!) step_a, Tensor boundaries_a, Tensor values_a, int nb_a, float beta1_a, float beta2_a, Tensor(b!) alpha_a, Tensor(c!) step_b, "
         "Tensor boundaries_b, Tensor values_b, int nb_b, float beta1_b, float beta2_b, Tensor(d!) alpha_b, Tensor(e!)? zero) -> ()", adam_schedule2);

@@ -13,6 +13,7 @@
 // Weight gradients are accumulated with fp32 atomics into one buffer per network (what the NCCL
 // all-reduce of the data-parallel path sums across GPUs).
 #include "common.cuh"
+#include "det.cuh"
 #include "mlp.cuh"
 #include "systems.cuh"
 
@@ -215,7 +216,8 @@ struct CriticSmem {
   float loss;
 };
 
-template <int S>
+// DET: grad is the partials workspace (det.cuh); the CTA adds into its slice, the loss partial included.
+template <int S, bool DET = false>
 __global__ void __launch_bounds__(UP_NT) k_critic_grad(const __grid_constant__ cacto_sys_params P, const float* __restrict__ cw,
                                                        const float* __restrict__ cwT, const float* __restrict__ tw, float w_S, int mc,
                                                        const float* __restrict__ state, const float* __restrict__ state_next,
@@ -227,6 +229,7 @@ __global__ void __launch_bounds__(UP_NT) k_critic_grad(const __grid_constant__ c
   extern __shared__ __align__(128) unsigned char smem_raw[];
   CriticSmem<S>& sm = *reinterpret_cast<CriticSmem<S>*>(smem_raw);
   const CriticLayout L(P.ns);
+  if constexpr (DET) grad += (size_t)blockIdx.x * det_stride(L.total);
   const int ns = P.ns, nx = P.nx, tid = threadIdx.x;
   const int64_t row0 = (int64_t)blockIdx.x * S;
   const int rows = (int)min((int64_t)S, B - row0);
@@ -356,10 +359,24 @@ __global__ void __launch_bounds__(UP_NT) k_critic_grad(const __grid_constant__ c
       sm.VBAR[tid] = vbar;
     }
     for (int off = 16; off > 0; off >>= 1) lsum += __shfl_xor_sync(0xffffffffu, lsum, off);
-    if ((tid & 31) == 0 && lsum != 0.f) atomicAdd(&sm.loss, lsum);
+    if constexpr (DET) {
+      // per-warp partials behind CriticSmem (launched with UP_NT / 32 more floats), summed in warp order
+      if ((tid & 31) == 0) reinterpret_cast<float*>(smem_raw + sizeof(CriticSmem<S>))[tid >> 5] = lsum;
+    } else {
+      if ((tid & 31) == 0 && lsum != 0.f) atomicAdd(&sm.loss, lsum);
+    }
   }
   __syncthreads();
-  if (tid == 0 && loss_out != nullptr) atomicAdd(loss_out, sm.loss);
+  if constexpr (DET) {
+    if (tid == 0) {
+      const float* lw = reinterpret_cast<const float*>(smem_raw + sizeof(CriticSmem<S>));
+      float l = 0.f;
+      for (int w = 0; w < UP_NT / 32; ++w) l += lw[w];
+      grad[L.total] += l;
+    }
+  } else {
+    if (tid == 0 && loss_out != nullptr) atomicAdd(loss_out, sm.loss);
+  }
 
   if (sobolev) {
     // ---- A: adjoint sweep through G (second-order terms); extra_l overwrites g_l, a_l kept for the outer products
@@ -381,7 +398,7 @@ __global__ void __launch_bounds__(UP_NT) k_critic_grad(const __grid_constant__ c
     __syncthreads();
     streamed<S, CR_H4>(pipe, sm, gi, &sm.A[0][koff(2)], CW, CR_H3, a_epi(3));
     __syncthreads();
-    tile_colsum<UP_NT>(&sm.A[0][koff(3)], CW, CR_H4, rows, grad + L.W[4]);       // d w5 += sum_s a_4
+    tile_colsum<UP_NT, DET>(&sm.A[0][koff(3)], CW, CR_H4, rows, grad + L.W[4]);       // d w5 += sum_s a_4
   } else {
     for (int i = tid; i < S * CW; i += UP_NT) sm.G[i / CW][i % CW] = 0.f;
     __syncthreads();
@@ -395,12 +412,12 @@ __global__ void __launch_bounds__(UP_NT) k_critic_grad(const __grid_constant__ c
   for (int o = tid; o < CR_H4; o += UP_NT) {                                                   // d w5 += sum_s vbar h_4
     float acc = 0.f;
     for (int s = 0; s < rows; ++s) acc += sm.VBAR[s] * sm.SN[s][koff(3) + o];
-    atomicAdd(grad + L.W[4] + o, acc);
+    grad_add<DET>(grad + L.W[4] + o, acc);
   }
   if (tid == 0) {
     float acc = 0.f;
     for (int s = 0; s < rows; ++s) acc += sm.VBAR[s];
-    atomicAdd(grad + L.b[4], acc);
+    grad_add<DET>(grad + L.b[4], acc);
   }
   __syncthreads();
   auto b_epi = [&](int l) {   // e_l = (e_{l+1} W_{l+1}^T) * cos z_l + extra_l
@@ -413,27 +430,27 @@ __global__ void __launch_bounds__(UP_NT) k_critic_grad(const __grid_constant__ c
   };
   const float* A2 = sobolev ? &sm.A[0][0] : nullptr;
   // layer 4
-  tile_outer2<S, CR_H4, UP_NT>(&sm.SN[0][koff(2)], CW, &sm.G[0][koff(3)], CW, A2 ? A2 + koff(2) : nullptr, CW, &sm.DL[0][koff(3)], CW,
+  tile_outer2<S, CR_H4, UP_NT, DET>(&sm.SN[0][koff(2)], CW, &sm.G[0][koff(3)], CW, A2 ? A2 + koff(2) : nullptr, CW, &sm.DL[0][koff(3)], CW,
                                CR_H3, grad + L.W[3], rows);
-  tile_colsum<UP_NT>(&sm.G[0][koff(3)], CW, CR_H4, rows, grad + L.b[3]);
+  tile_colsum<UP_NT, DET>(&sm.G[0][koff(3)], CW, CR_H4, rows, grad + L.b[3]);
   streamed<S, CR_H3>(pipe, sm, gi, &sm.G[0][koff(3)], CW, CR_H4, b_epi(2));
   __syncthreads();
   // layer 3
-  tile_outer2<S, CR_H3, UP_NT>(&sm.SN[0][koff(1)], CW, &sm.G[0][koff(2)], CW, A2 ? A2 + koff(1) : nullptr, CW, &sm.DL[0][koff(2)], CW,
+  tile_outer2<S, CR_H3, UP_NT, DET>(&sm.SN[0][koff(1)], CW, &sm.G[0][koff(2)], CW, A2 ? A2 + koff(1) : nullptr, CW, &sm.DL[0][koff(2)], CW,
                                CR_H2, grad + L.W[2], rows);
-  tile_colsum<UP_NT>(&sm.G[0][koff(2)], CW, CR_H3, rows, grad + L.b[2]);
+  tile_colsum<UP_NT, DET>(&sm.G[0][koff(2)], CW, CR_H3, rows, grad + L.b[2]);
   streamed<S, CR_H2>(pipe, sm, gi, &sm.G[0][koff(2)], CW, CR_H3, b_epi(1));
   __syncthreads();
   // layer 2
-  tile_outer2<S, CR_H2, UP_NT>(&sm.SN[0][koff(0)], CW, &sm.G[0][koff(1)], CW, A2 ? A2 + koff(0) : nullptr, CW, &sm.DL[0][koff(1)], CW,
+  tile_outer2<S, CR_H2, UP_NT, DET>(&sm.SN[0][koff(0)], CW, &sm.G[0][koff(1)], CW, A2 ? A2 + koff(0) : nullptr, CW, &sm.DL[0][koff(1)], CW,
                                CR_H1, grad + L.W[1], rows);
-  tile_colsum<UP_NT>(&sm.G[0][koff(1)], CW, CR_H2, rows, grad + L.b[1]);
+  tile_colsum<UP_NT, DET>(&sm.G[0][koff(1)], CW, CR_H2, rows, grad + L.b[1]);
   streamed<S, CR_H1>(pipe, sm, gi, &sm.G[0][koff(1)], CW, CR_H2, b_epi(0));
   __syncthreads();
   // layer 1
-  tile_outer2<S, CR_H1, UP_NT>(&XN[0][0], NSP, &sm.G[0][koff(0)], CW, sobolev ? &sm.A0[0][0] : nullptr, NSP, &sm.DL[0][koff(0)], CW, ns,
+  tile_outer2<S, CR_H1, UP_NT, DET>(&XN[0][0], NSP, &sm.G[0][koff(0)], CW, sobolev ? &sm.A0[0][0] : nullptr, NSP, &sm.DL[0][koff(0)], CW, ns,
                                grad + L.W[0], rows);
-  tile_colsum<UP_NT>(&sm.G[0][koff(0)], CW, CR_H1, rows, grad + L.b[0]);
+  tile_colsum<UP_NT, DET>(&sm.G[0][koff(0)], CW, CR_H1, rows, grad + L.b[0]);
 }
 
 // ------------------------------------------------------------------------------------------ actor
@@ -454,7 +471,7 @@ struct ActorSmem {
   float ACT[S][NAP], D3[S][NAP], DRDA[S][NAP];
 };
 
-template <int SYS, int S>
+template <int SYS, int S, bool DET = false>
 __global__ void __launch_bounds__(UP_NT) k_actor_grad(const __grid_constant__ cacto_sys_params P, const float* __restrict__ aw,
                                                       const float* __restrict__ awT, const float* __restrict__ cw,
                                                       const float* __restrict__ cwT, const float* __restrict__ state,
@@ -466,6 +483,7 @@ __global__ void __launch_bounds__(UP_NT) k_actor_grad(const __grid_constant__ ca
   ActorSmem<S>& sm = *reinterpret_cast<ActorSmem<S>*>(smem_raw);
   const ActorLayout LA(NS, NA);
   const CriticLayout LC(NS);
+  if constexpr (DET) grad += (size_t)blockIdx.x * det_stride(LA.total);
   const int tid = threadIdx.x;
   const int64_t row0 = (int64_t)blockIdx.x * S;
   const int rows = (int)min((int64_t)S, B - row0);
@@ -608,12 +626,12 @@ __global__ void __launch_bounds__(UP_NT) k_actor_grad(const __grid_constant__ ca
     const int k = i / NA, j = i - k * NA;
     float acc = 0.f;
     for (int s = 0; s < rows; ++s) acc = fmaf(sm.H2[s][k], sm.D3[s][j], acc);
-    atomicAdd(grad + LA.W3 + i, acc);
+    grad_add<DET>(grad + LA.W3 + i, acc);
   }
   if (tid < NA) {
     float acc = 0.f;
     for (int s = 0; s < rows; ++s) acc += sm.D3[s][tid];
-    atomicAdd(grad + LA.b3 + tid, acc);
+    grad_add<DET>(grad + LA.b3 + tid, acc);
   }
   for (int i = tid; i < S * ACTOR_H; i += UP_NT) {             // e2 = (d3 W3^T) * lrelu'(z2)
     const int s = i / ACTOR_H, n = i - s * ACTOR_H;
@@ -623,8 +641,8 @@ __global__ void __launch_bounds__(UP_NT) k_actor_grad(const __grid_constant__ ca
     sm.E[s][n] = acc * (sm.H2[s][n] > 0.f ? 1.f : LEAKY_ALPHA);
   }
   __syncthreads();
-  tile_outer2<S, ACTOR_H, UP_NT>(&sm.H1[0][0], ACTOR_H, &sm.E[0][0], ACTOR_H, nullptr, 0, nullptr, 0, ACTOR_H, grad + LA.W2, rows);
-  tile_colsum<UP_NT>(&sm.E[0][0], ACTOR_H, ACTOR_H, rows, grad + LA.b2);
+  tile_outer2<S, ACTOR_H, UP_NT, DET>(&sm.H1[0][0], ACTOR_H, &sm.E[0][0], ACTOR_H, nullptr, 0, nullptr, 0, ACTOR_H, grad + LA.W2, rows);
+  tile_colsum<UP_NT, DET>(&sm.E[0][0], ACTOR_H, ACTOR_H, rows, grad + LA.b2);
   streamed<S, ACTOR_H>(pipe, sm, gi, &sm.E[0][0], ACTOR_H, ACTOR_H, [&](int r, int c, const float4& a) {
     const float4 h = *reinterpret_cast<const float4*>(&sm.H1[r][c]);
     *reinterpret_cast<float4*>(&sm.H2[r][c]) =
@@ -632,8 +650,8 @@ __global__ void __launch_bounds__(UP_NT) k_actor_grad(const __grid_constant__ ca
                     a.w * (h.w > 0.f ? 1.f : LEAKY_ALPHA));
   });
   __syncthreads();
-  tile_outer2<S, ACTOR_H, UP_NT>(&sm.XN[0][0], NSP, &sm.H2[0][0], ACTOR_H, nullptr, 0, nullptr, 0, NS, grad + LA.W1, rows);
-  tile_colsum<UP_NT>(&sm.H2[0][0], ACTOR_H, ACTOR_H, rows, grad + LA.b1);
+  tile_outer2<S, ACTOR_H, UP_NT, DET>(&sm.XN[0][0], NSP, &sm.H2[0][0], ACTOR_H, nullptr, 0, nullptr, 0, NS, grad + LA.W1, rows);
+  tile_colsum<UP_NT, DET>(&sm.H2[0][0], ACTOR_H, ACTOR_H, rows, grad + LA.b1);
 }
 
 // ------------------------------------------------------------------------------------------ forward-only kernels
@@ -1005,6 +1023,145 @@ extern "C" int cacto_actor_grad(const cacto_sys_params* p, const float* actor_pa
     case CACTO_CAR_PARK: return launch_actor_grad<CACTO_CAR_PARK>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, st);
     case CACTO_MANIPULATOR: return launch_actor_grad<CACTO_MANIPULATOR>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, st);
     case CACTO_UR5: return launch_actor_grad<CACTO_UR5>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, st);
+    default: return CACTO_E_SYSTEM;
+  }
+}
+
+// ---- deterministic variants (det.cuh): the same kernels with DET = true, in waves of at most CACTO_DET_MAX_SLICES CTAs
+namespace cacto {
+
+__global__ void __launch_bounds__(256) k_det_reduce(const float* __restrict__ part, int64_t slices, int64_t stride, int64_t n,
+                                                    float* __restrict__ grad, float* __restrict__ loss) {
+  pdl_wait();
+  const int64_t i = (int64_t)blockIdx.x * blockDim.x + threadIdx.x;
+  if (i > n || (i == n && loss == nullptr)) return;
+  float s = 0.f;
+  for (int64_t j = 0; j < slices; ++j) s += part[j * stride + i];
+  if (i < n) grad[i] += s;
+  else loss[0] += s;
+}
+
+int det_reduce(const float* part, int64_t slices, int64_t n, float* grad, float* loss, cudaStream_t st) {
+  if (cudaError_t le = launch_pdl(k_det_reduce, (unsigned)((n + 1 + 255) / 256), 256, 0, st, part, slices, det_stride(n), n, grad, loss)) return (int)le;
+  CACTO_LAUNCH_CHECK();
+  return 0;
+}
+
+static bool partials_ok(int64_t have, int64_t need) { return need >= 0 && have >= need; }
+
+template <int S>
+static int critic_grad_det_s(const cacto_sys_params& P, const float* cw, const float* cwT, const float* tw, float w_S, int mc, const float* state,
+                             const float* state_next, const float* prtg, const float* dVdx, const float* done, const float* weights, float inv_B,
+                             float* grad, float* rtg, float* V, float* Vt, float* loss, int64_t B, float* part, cudaStream_t st) {
+  auto k = k_critic_grad<S, true>;
+  const size_t smem = sizeof(CriticSmem<S>) + (UP_NT / 32) * sizeof(float);
+  if (int e = smem_attr(k, smem)) return e;
+  const int64_t n = CriticLayout(P.ns).total, tiles = (B + S - 1) / S, slices = det_slices(tiles), ns = P.ns;
+  if (cudaError_t e = cudaMemsetAsync(part, 0, (size_t)(slices * det_stride(n)) * sizeof(float), st)) return (int)e;
+  for (int64_t t0 = 0; t0 < tiles; t0 += slices) {
+    const int64_t r0 = t0 * S, rows = min(B - r0, slices * S);
+    if (cudaError_t le = launch_pdl(k, (unsigned)((rows + S - 1) / S), UP_NT, smem, st, P, cw, cwT, tw, w_S, mc, state + r0 * ns,
+                                    state_next ? state_next + r0 * ns : nullptr, prtg + r0, dVdx ? dVdx + r0 * ns : nullptr, done ? done + r0 : nullptr,
+                                    weights + r0, inv_B, part, rtg + r0, V + r0, Vt + r0, loss, rows))
+      return (int)le;
+    CACTO_LAUNCH_CHECK();
+  }
+  return det_reduce(part, slices, n, grad, loss, st);
+}
+
+template <int SYS, int S>
+static int actor_grad_det_s(const cacto_sys_params& P, const float* aw, const float* awT, const float* cw, const float* cwT, const float* state,
+                            const double* term, float inv_B, float* grad, float* actions, int64_t B, float* part, cudaStream_t st) {
+  auto k = k_actor_grad<SYS, S, true>;
+  if (int e = smem_attr(k, sizeof(ActorSmem<S>))) return e;
+  const int64_t n = ActorLayout(P.ns, P.na).total, tiles = (B + S - 1) / S, slices = det_slices(tiles), ns = P.ns, na = P.na;
+  if (cudaError_t e = cudaMemsetAsync(part, 0, (size_t)(slices * det_stride(n)) * sizeof(float), st)) return (int)e;
+  for (int64_t t0 = 0; t0 < tiles; t0 += slices) {
+    const int64_t r0 = t0 * S, rows = min(B - r0, slices * S);
+    if (cudaError_t le = launch_pdl(k, (unsigned)((rows + S - 1) / S), UP_NT, sizeof(ActorSmem<S>), st, P, aw, awT, cw, cwT, state + r0 * ns, term + r0,
+                                    inv_B, part, actions ? actions + r0 * na : nullptr, rows))
+      return (int)le;
+    CACTO_LAUNCH_CHECK();
+  }
+  return det_reduce(part, slices, n, grad, nullptr, st);
+}
+
+template <int SYS>
+static int actor_grad_det(const cacto_sys_params& P, const float* aw, const float* awT, const float* cw, const float* cwT, const float* state,
+                          const double* term, float inv_B, float* grad, float* actions, int64_t B, float* part, cudaStream_t st) {
+  switch (pick_tile(B)) {
+    case 16: return actor_grad_det_s<SYS, 16>(P, aw, awT, cw, cwT, state, term, inv_B, grad, actions, B, part, st);
+    case 8: return actor_grad_det_s<SYS, 8>(P, aw, awT, cw, cwT, state, term, inv_B, grad, actions, B, part, st);
+    case 4: return actor_grad_det_s<SYS, 4>(P, aw, awT, cw, cwT, state, term, inv_B, grad, actions, B, part, st);
+    default: return actor_grad_det_s<SYS, 2>(P, aw, awT, cw, cwT, state, term, inv_B, grad, actions, B, part, st);
+  }
+}
+
+}  // namespace cacto
+
+extern "C" int64_t cacto_det_partials_floats(int32_t net, int64_t B, int32_t ns, int32_t na, int32_t nh1, int32_t nh2) {
+  if (B < 0 || ns < 2 || ns > CACTO_MAX_NS || na < 1 || na > CACTO_MAX_NA) return CACTO_E_SIZE;
+  int64_t n, tile;
+  switch (net) {
+    case CACTO_DET_CRITIC: n = CriticLayout(ns).total; tile = pick_tile(B); break;
+    case CACTO_DET_ACTOR: n = ActorLayout(ns, na).total; tile = pick_tile(B); break;
+    case CACTO_DET_ACTOR_WIDTH:
+      if (nh1 < 1 || nh1 > CACTO_ACTOR_MAX_WIDTH || nh2 < 1 || nh2 > CACTO_ACTOR_MAX_WIDTH) return CACTO_E_SIZE;
+      n = ActorLayout(ns, na, nh1, nh2).total; tile = actor_width_tile(B); break;
+    case CACTO_DET_CRITIC_TC:      // tcgen05 engine: 3 / 2 regions of fixed-size slices, one per CTA of a <= 296-CTA grid over 128-sample tiles
+    case CACTO_DET_ACTOR_TC: return (net == CACTO_DET_CRITIC_TC ? 3 : 2) * det_slices((B + 127) / 128) * det_tc_slice;
+    default: return CACTO_E_SIZE;
+  }
+  return det_slices((B + tile - 1) / tile) * det_stride(n);
+}
+
+extern "C" int cacto_critic_grad_det(const cacto_sys_params* p, const float* critic_params, const float* critic_params_T,
+                                     const float* target_params, float w_S, int mc, const float* state, const float* state_next,
+                                     const float* partial_rtg, const float* dVdx, const float* done, const float* weights, float inv_B,
+                                     float* grad, float* rtg, float* V, float* V_target_s, float* loss, int64_t B, float* partials,
+                                     int64_t partials_floats, void* stream) {
+  if (!p) return CACTO_E_ARG;
+  if (B < 0) return CACTO_E_SIZE;
+  if (B == 0) return 0;
+  if (!critic_params || !critic_params_T || !target_params || !state || !partial_rtg || !weights || !grad || !rtg || !V || !V_target_s || !partials)
+    return CACTO_E_ARG;
+  if (!mc && (!state_next || !done)) return CACTO_E_ARG;
+  if (w_S != 0.f && !dVdx) return CACTO_E_ARG;
+  if (!aligned16(critic_params) || !aligned16(critic_params_T) || !aligned16(target_params) || !aligned16(grad) || !aligned16(partials))
+    return CACTO_E_ALIGN;
+  if (!partials_ok(partials_floats, cacto_det_partials_floats(CACTO_DET_CRITIC, B, p->ns, p->na, 0, 0))) return CACTO_E_SIZE;
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (pick_tile(B)) {
+    case 16: return critic_grad_det_s<16>(*p, critic_params, critic_params_T, target_params, w_S, mc, state, state_next, partial_rtg, dVdx, done, weights,
+                                          inv_B, grad, rtg, V, V_target_s, loss, B, partials, st);
+    case 8: return critic_grad_det_s<8>(*p, critic_params, critic_params_T, target_params, w_S, mc, state, state_next, partial_rtg, dVdx, done, weights,
+                                        inv_B, grad, rtg, V, V_target_s, loss, B, partials, st);
+    case 4: return critic_grad_det_s<4>(*p, critic_params, critic_params_T, target_params, w_S, mc, state, state_next, partial_rtg, dVdx, done, weights,
+                                        inv_B, grad, rtg, V, V_target_s, loss, B, partials, st);
+    default: return critic_grad_det_s<2>(*p, critic_params, critic_params_T, target_params, w_S, mc, state, state_next, partial_rtg, dVdx, done, weights,
+                                         inv_B, grad, rtg, V, V_target_s, loss, B, partials, st);
+  }
+}
+
+extern "C" int cacto_actor_grad_det(const cacto_sys_params* p, const float* actor_params, const float* actor_params_T,
+                                    const float* critic_params, const float* critic_params_T, const float* state, const double* term,
+                                    float inv_B, float* grad, float* actions, int64_t B, float* partials, int64_t partials_floats, void* stream) {
+  if (!p) return CACTO_E_ARG;
+  if (B < 0) return CACTO_E_SIZE;
+  if (B == 0) return 0;
+  if (!actor_params || !actor_params_T || !critic_params || !critic_params_T || !state || !term || !grad || !partials) return CACTO_E_ARG;
+  if (!aligned16(actor_params) || !aligned16(actor_params_T) || !aligned16(critic_params) || !aligned16(critic_params_T) || !aligned16(grad) ||
+      !aligned16(partials))
+    return CACTO_E_ALIGN;
+  if (!partials_ok(partials_floats, cacto_det_partials_floats(CACTO_DET_ACTOR, B, p->ns, p->na, 0, 0))) return CACTO_E_SIZE;
+  cudaStream_t st = (cudaStream_t)stream;
+  switch (p->system) {
+    case CACTO_SINGLE_INTEGRATOR: return actor_grad_det<CACTO_SINGLE_INTEGRATOR>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, partials, st);
+    case CACTO_DOUBLE_INTEGRATOR: return actor_grad_det<CACTO_DOUBLE_INTEGRATOR>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, partials, st);
+    case CACTO_CAR: return actor_grad_det<CACTO_CAR>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, partials, st);
+    case CACTO_CAR_PARK: return actor_grad_det<CACTO_CAR_PARK>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, partials, st);
+    case CACTO_MANIPULATOR: return actor_grad_det<CACTO_MANIPULATOR>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, partials, st);
+    case CACTO_UR5: return actor_grad_det<CACTO_UR5>(*p, actor_params, actor_params_T, critic_params, critic_params_T, state, term, inv_B, grad, actions, B, partials, st);
     default: return CACTO_E_SYSTEM;
   }
 }

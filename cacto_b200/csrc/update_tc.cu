@@ -16,6 +16,7 @@
 //   k_tc_actor_bwd    actor backward;                 k_tc_wgrad      all weight gradients of a step in one launch
 #include <string.h>
 #include "common.cuh"
+#include "det.cuh"
 #include "mlp.cuh"
 #include "systems.cuh"
 #include "tc_common.cuh"
@@ -94,6 +95,37 @@ struct TcWs {
 };
 enum { ST_TF = 0, ST_CF, ST_CB, ST_AF, ST_AB };
 constexpr int WG_MAX_CTAS = 192;
+
+// ---- deterministic variants (DET = true; cacto_*_grad_tc_det).  The bias / head column sums and the loss are the only cross-warp and
+// cross-CTA float sums of the chain kernels (the weight matrices already go through the fixed-order k_tc_wgrad_reduce).  With DET
+// every epilogue quadrant q sums into its own copy colq[q] of the column sums (behind the chain's shared state, TC_DET_SMEM bytes;
+// one warp per entry), the loss per warp into lossw[warp]; at the end the CTA writes (colq[0] + colq[1]) + (colq[2] + colq[3]) and
+// the warp-ordered loss into its slice of a partials region -- every entry of the slice, so the region needs no clearing -- and
+// k_tc_det_reduce adds the slices of each region into grad in slice order.  Slice layout (TC_DET_SLICE floats), critic: [0, 384) d b_l
+// at kofs(l), [384, 512) d w5, 512 d b5, TC_DET_LOSS the loss; actor: [0, 256) d b2, [256, 512) d b1, [512, 512 + na) d b3.
+constexpr int TC_DET_SLICE = (int)det_tc_slice, TC_DET_LOSS = 640, TC_DET_COLS = 640;
+constexpr size_t TC_DET_SMEM = (4 * TC_DET_COLS + EPI_WARPS) * sizeof(float);
+template <typename SM>
+__device__ __forceinline__ float* det_colq(unsigned char* smem_raw) { return reinterpret_cast<float*>(smem_raw + sizeof(SM)); }
+template <typename SM>
+__device__ __forceinline__ void det_clear(unsigned char* smem_raw, int tid) {        // before chain_setup (whose barrier publishes it)
+  float* q = det_colq<SM>(smem_raw);
+  for (int i = tid; i < 4 * TC_DET_COLS + EPI_WARPS; i += THREADS) q[i] = 0.f;
+}
+// epilogue threads, after the epi_bar that ends the jobs: column sums [0, n) go to slice entries [dst, dst + n)
+template <typename SM>
+__device__ __forceinline__ void det_flush(unsigned char* smem_raw, float* slice, int n, int dst, bool loss, int tid) {
+  const float* q = det_colq<SM>(smem_raw);
+  for (int i = tid; i < TC_DET_SLICE; i += EPI_THREADS) {
+    float v = 0.f;
+    const int k = i - dst;
+    if (k >= 0 && k < n) v = (q[k] + q[TC_DET_COLS + k]) + (q[2 * TC_DET_COLS + k] + q[3 * TC_DET_COLS + k]);
+    if (i == TC_DET_LOSS && loss) {
+      for (int w = 0; w < EPI_WARPS; ++w) v += q[4 * TC_DET_COLS + w];
+    }
+    slice[i] = v;
+  }
+}
 
 static LayerSeq seq_critic_fwd() { LayerSeq L = {4, {16, CR_H1, CR_H2, CR_H3}, {CR_H1, CR_H2, CR_H3, CR_H4}}; return L; }
 static LayerSeq seq_critic_bwd(int n) { LayerSeq L = {n, {CR_H4, CR_H3, CR_H2, CR_H1}, {CR_H3, CR_H2, CR_H1, 16}}; return L; }
@@ -381,12 +413,14 @@ struct BwdArgs {
 // These sweeps do little arithmetic per element; what they wait for is the workspace (cos z, extra, g, sin z: L2 / HBM latency)
 // and the accumulator.  Every layer therefore issues the loads of ALL its workspace operands before it waits for the MMAs
 // (they do not depend on them), so that the two latencies overlap instead of adding up.
-template <int MODE>
+// DET: A.grad is the kernel's partials region; CTA j writes slice j.
+template <int MODE, bool DET = false>
 __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_bwd(const __grid_constant__ cacto_sys_params P, const BwdArgs A, const TcWs ws, const LayerSeq L,
                                                               int njobs) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   CriticSmemTc& sm = *reinterpret_cast<CriticSmemTc*>(smem_raw);
   const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
+  if constexpr (DET) det_clear<CriticSmemTc>(smem_raw, tid);
   chain_setup(sm, tid, warp);
   pdl_wait();            // everything above overlaps the tail of the preceding kernel (programmatic dependent launch)
   const uint32_t tmem = sm.tmem_base;
@@ -394,6 +428,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_bwd(const __grid_const
   const ActorLayout AL(P.ns, P.na);
   if (warp < EPI_WARPS) {
     Epi e = epi_init(tid, tmem);
+    float* const colsum = DET ? det_colq<CriticSmemTc>(smem_raw) + TC_DET_COLS * e.q : sm.colsum;
     TCU_TRACE_DECL;
 #define EEV(code) do { if (tid == 0) TCU_EV(0, code); } while (0)
     const float* US = ws.US + 8 * ST_CB;
@@ -459,7 +494,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_bwd(const __grid_const
             m = fmaxf(m, fabsf(ev[j][i]));
           }
           ws_store16(ws.EE, CWT, tile, kofs(3) + 16 * ch, e.row, ev[j]);
-          warp_colsum16(sm.colsum, kofs(3) + 16 * ch, ev[j], e.lane);           // d b_4
+          warp_colsum16<DET>(colsum, kofs(3) + 16 * ch, ev[j], e.lane);           // d b_4
         }
         // d w5 += sum_s vbar h_4 is a batch reduction like the other weight gradients: vbar goes to the workspace as a 4-wide
         // tensor (column 0) and k_tc_wgrad pairs it with sin z_4
@@ -471,7 +506,10 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_bwd(const __grid_const
           float t = vb;
 #pragma unroll
           for (int o = 16; o > 0; o >>= 1) t += __shfl_xor_sync(0xffffffffu, t, o);
-          if (e.lane == 0) atomicAdd(&sm.colsum[CWT + CR_H4], t);
+          if (e.lane == 0) {
+            if constexpr (DET) colsum[CWT + CR_H4] += t;
+            else atomicAdd(&sm.colsum[CWT + CR_H4], t);
+          }
         }
         amax_update(ws.amax + AM_EE, m, e.lane);
         m = row_max4(sm, e, m);
@@ -523,7 +561,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_bwd(const __grid_const
 #pragma unroll
               for (int i = 0; i < 16; ++i) v[i] = vz * (v[i] * us * c[j][i] + (sob ? x[i] : 0.f));
               ws_store16(ws.EE, CWT, tile, col0 + 16 * ch, e.row, v);
-              warp_colsum16(sm.colsum, col0 + 16 * ch, v, e.lane);                   // d b_l
+              warp_colsum16<DET>(colsum, col0 + 16 * ch, v, e.lane);                   // d b_l
             } else {
 #pragma unroll
               for (int i = 0; i < 16; ++i) v[i] *= us;
@@ -601,7 +639,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_bwd(const __grid_const
             }
             ws_store16(ws.D3, 16, tile, 0, e.row, d3);
             amax_update(ws.amax + AM_D3, m, e.lane);
-            warp_colsum16(sm.colsum, 0, d3, e.lane);                     // d b3
+            warp_colsum16<DET>(colsum, 0, d3, e.lane);                     // d b3
           }
         }
       }
@@ -610,10 +648,19 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_bwd(const __grid_const
     if (MODE == BWD_G || MODE == BWD_B) {
 #pragma unroll
       for (int o = 16; o > 0; o >>= 1) lsum += __shfl_xor_sync(0xffffffffu, lsum, o);
-      if (e.lane == 0 && lsum != 0.f && A.loss_out != nullptr) atomicAdd(A.loss_out, lsum);
+      if constexpr (DET) {
+        if (e.lane == 0) det_colq<CriticSmemTc>(smem_raw)[4 * TC_DET_COLS + e.warp] = lsum;
+      } else {
+        if (e.lane == 0 && lsum != 0.f && A.loss_out != nullptr) atomicAdd(A.loss_out, lsum);
+      }
     }
     epi_bar();
-    if (MODE == BWD_B) {
+    if constexpr (DET) {
+      float* slice = A.grad + (int64_t)blockIdx.x * TC_DET_SLICE;
+      if (MODE == BWD_B) det_flush<CriticSmemTc>(smem_raw, slice, CWT + CR_H4 + 1, 0, true, tid);
+      else if (MODE == BWD_G) det_flush<CriticSmemTc>(smem_raw, slice, 0, 0, true, tid);
+      else det_flush<CriticSmemTc>(smem_raw, slice, P.na, 2 * ACTOR_H, false, tid);
+    } else if (MODE == BWD_B) {
       for (int i = tid; i < CWT + CR_H4 + 1; i += EPI_THREADS) {
         const float v = sm.colsum[i];
         if (v == 0.f) continue;
@@ -641,17 +688,20 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_bwd(const __grid_const
 }
 
 // ================================================================================================== adjoint sweep (A)
+template <bool DET = false>     // DET: grad is the kernel's partials region; CTA j writes slice j
 __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_adj(const __grid_constant__ cacto_sys_params P, const float* __restrict__ critic, float* __restrict__ grad,
                                                               const TcWs ws, const LayerSeq L, int njobs, int64_t B) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   CriticSmemTc& sm = *reinterpret_cast<CriticSmemTc*>(smem_raw);
   const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
+  if constexpr (DET) det_clear<CriticSmemTc>(smem_raw, tid);
   chain_setup(sm, tid, warp);
   pdl_wait();            // everything above overlaps the tail of the preceding kernel (programmatic dependent launch)
   const uint32_t tmem = sm.tmem_base;
   const CriticLayout CL(P.ns);
   if (warp < EPI_WARPS) {
     Epi e = epi_init(tid, tmem);
+    float* const colsum = DET ? det_colq<CriticSmemTc>(smem_raw) + TC_DET_COLS * e.q : sm.colsum;
     const float* US = ws.US + 8 * ST_CF;
     const float* w5 = critic + CL.W[4];
     for (int job = blockIdx.x; job < njobs; job += gridDim.x) {
@@ -716,7 +766,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_adj(const __grid_const
               put_a16(sm, e, 16 * ch, v, s);
               publish_a_group(sm, j);
             } else {
-              warp_colsum16(sm.colsum, 16 * ch, v, e.lane);                  // d w5 += sum_s a_4
+              warp_colsum16<DET>(colsum, 16 * ch, v, e.lane);                  // d w5 += sum_s a_4
             }
           }
         if (l < 3) amax_update(ws.amax + AM_AA, am, e.lane);
@@ -727,7 +777,8 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_critic_adj(const __grid_const
       }
     }
     epi_bar();
-    if (tid < CR_H4 && sm.colsum[tid] != 0.f) atomicAdd(grad + CL.W[4] + tid, sm.colsum[tid]);
+    if constexpr (DET) det_flush<CriticSmemTc>(smem_raw, grad + (int64_t)blockIdx.x * TC_DET_SLICE, CR_H4, CWT, false, tid);
+    else if (tid < CR_H4 && sm.colsum[tid] != 0.f) atomicAdd(grad + CL.W[4] + tid, sm.colsum[tid]);
   } else if (warp == EPI_WARPS) {
     RingState rs = {0, 0u, 0u};
     int tcu_trace_n = 0;
@@ -854,17 +905,20 @@ __global__ void __launch_bounds__(128) k_tc_actor_env(const __grid_constant__ ca
   for (int j = 0; j < NA; ++j) ws.DRDA[b * NA + j] = g[j];
 }
 
+template <bool DET = false>     // DET: grad is the kernel's partials region; CTA j writes slice j
 __global__ void __launch_bounds__(THREADS, 1) k_tc_actor_bwd(const __grid_constant__ cacto_sys_params P, float* __restrict__ grad, const TcWs ws,
                                                              const LayerSeq L, int njobs, int64_t B) {
   extern __shared__ __align__(1024) unsigned char smem_raw[];
   ActorSmemTc& sm = *reinterpret_cast<ActorSmemTc*>(smem_raw);
   const int tid = threadIdx.x, warp = __shfl_sync(0xffffffffu, tid >> 5, 0);
+  if constexpr (DET) det_clear<ActorSmemTc>(smem_raw, tid);
   chain_setup(sm, tid, warp);
   pdl_wait();            // everything above overlaps the tail of the preceding kernel (programmatic dependent launch)
   const uint32_t tmem = sm.tmem_base;
   const ActorLayout AL(P.ns, P.na);
   if (warp < EPI_WARPS) {
     Epi e = epi_init(tid, tmem);
+    float* const colsum = DET ? det_colq<ActorSmemTc>(smem_raw) + TC_DET_COLS * e.q : sm.colsum;
     const float* US = ws.US + 8 * ST_AB;
     for (int job = blockIdx.x; job < njobs; job += gridDim.x) {
       const int64_t tile = job, b = tile * TILE + e.row;
@@ -911,7 +965,7 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_actor_bwd(const __grid_consta
             mx = fmaxf(mx, fabsf(v[i]));
           }
           ws_store16(Ep, ACTOR_H, tile, 16 * ch, e.row, v);
-          warp_colsum16(sm.colsum, l * ACTOR_H + 16 * ch, v, e.lane);        // d b2 | d b1
+          warp_colsum16<DET>(colsum, l * ACTOR_H + 16 * ch, v, e.lane);        // d b2 | d b1
           if (l == 0) {
             put_a16(sm, e, 16 * ch, v, s);
             publish_a_group(sm, j);
@@ -922,9 +976,13 @@ __global__ void __launch_bounds__(THREADS, 1) k_tc_actor_bwd(const __grid_consta
       }
     }
     epi_bar();
-    for (int i = tid; i < 2 * ACTOR_H; i += EPI_THREADS) {
-      const float v = sm.colsum[i];
-      if (v != 0.f) atomicAdd(grad + (i < ACTOR_H ? AL.b2 + i : AL.b1 + (i - ACTOR_H)), v);
+    if constexpr (DET) {
+      det_flush<ActorSmemTc>(smem_raw, grad + (int64_t)blockIdx.x * TC_DET_SLICE, 2 * ACTOR_H, 0, false, tid);
+    } else {
+      for (int i = tid; i < 2 * ACTOR_H; i += EPI_THREADS) {
+        const float v = sm.colsum[i];
+        if (v != 0.f) atomicAdd(grad + (i < ACTOR_H ? AL.b2 + i : AL.b1 + (i - ACTOR_H)), v);
+      }
     }
   } else if (warp == EPI_WARPS) {
     RingState rs = {0, 0u, 0u};
@@ -1212,6 +1270,39 @@ __global__ void __launch_bounds__(256) k_tc_wgrad_reduce(const WgTable T, const 
   if (c + 3 < J.N_real) o[3 * J.ldn] += acc.w;
 }
 
+// grad[map(i)] += sum_j part[r][j][i] for each region r in order (slices j in order, from 0.0f); the loss entry into loss[0]
+__global__ void __launch_bounds__(256) k_tc_det_reduce(const float* __restrict__ part, int regions, int slices, int is_critic, int ns, int na,
+                                                       float* __restrict__ grad, float* __restrict__ loss) {
+  pdl_wait();
+  const int i = blockIdx.x * blockDim.x + threadIdx.x;
+  if (i >= TC_DET_SLICE) return;
+  int64_t g = -1;
+  if (is_critic) {
+    const CriticLayout CL(ns);
+    if (i < CWT) {
+      const int l = i < kofs(1) ? 0 : (i < kofs(2) ? 1 : (i < kofs(3) ? 2 : 3));
+      g = CL.b[l] + (i - kofs(l));
+    } else if (i < CWT + CR_H4) {
+      g = CL.W[4] + (i - CWT);
+    } else if (i == CWT + CR_H4) {
+      g = CL.b[4];
+    }
+  } else {
+    const ActorLayout AL(ns, na);
+    if (i < ACTOR_H) g = AL.b2 + i;
+    else if (i < 2 * ACTOR_H) g = AL.b1 + (i - ACTOR_H);
+    else if (i < 2 * ACTOR_H + na) g = AL.b3 + (i - 2 * ACTOR_H);
+  }
+  const bool is_loss = is_critic && i == TC_DET_LOSS && loss != nullptr;
+  if (g < 0 && !is_loss) return;
+  for (int r = 0; r < regions; ++r) {
+    float s = 0.f;
+    for (int j = 0; j < slices; ++j) s += part[((int64_t)r * slices + j) * TC_DET_SLICE + i];
+    if (g >= 0) grad[g] += s;
+    else loss[0] += s;
+  }
+}
+
 // ================================================================================================== host side
 static int64_t align_up(int64_t x, int64_t a) { return (x + a - 1) / a * a; }
 // every kernel of the update chain is launched with the programmatic-serialization attribute and calls pdl_wait() (common.cuh)
@@ -1336,6 +1427,9 @@ static int launch_wgrad(WgTable& WT, const TcWs& ws, int sms, cudaStream_t st) {
   CACTO_LAUNCH_CHECK();
   return 0;
 }
+// the deterministic variants have one partials slice per CTA: at most CACTO_DET_MAX_SLICES of them
+template <bool DET>
+static int det_grid(int grid) { return DET && grid > CACTO_DET_MAX_SLICES ? CACTO_DET_MAX_SLICES : grid; }
 static WgOperand wg_op(const float* p, int W, int c0, int amax) { WgOperand o = {p, W, c0, amax}; return o; }
 
 template <int SYS>
@@ -1358,10 +1452,11 @@ extern "C" int64_t cacto_update_tc_workspace_bytes(int64_t B, int32_t ns, int32_
   return tc_ws_layout(nullptr, B, ns, na, nullptr);
 }
 
-extern "C" int cacto_critic_grad_tc(const cacto_sys_params* p, const float* critic_params, const float* target_params, float w_S, int mc,
+template <bool DET>
+static int critic_grad_tc(const cacto_sys_params* p, const float* critic_params, const float* target_params, float w_S, int mc,
                                     const float* state, const float* state_next, const float* partial_rtg, const float* dVdx, const float* done,
                                     const float* weights, float inv_B, float* grad, float* rtg, float* V, float* V_target_s, float* loss, int64_t B,
-                                    void* workspace, int64_t workspace_bytes, void* stream) {
+                                    void* workspace, int64_t workspace_bytes, float* part, int64_t part_floats, void* stream) {
   if (!p) return CACTO_E_ARG;
   if (B < 0) return CACTO_E_SIZE;
   if (B == 0) return 0;
@@ -1370,6 +1465,12 @@ extern "C" int cacto_critic_grad_tc(const cacto_sys_params* p, const float* crit
   if (w_S != 0.f && !dVdx) return CACTO_E_ARG;
   if ((reinterpret_cast<uintptr_t>(workspace) & 255) || (reinterpret_cast<uintptr_t>(grad) & 15) || (reinterpret_cast<uintptr_t>(critic_params) & 15))
     return CACTO_E_ALIGN;
+  if (DET) {
+    if (!part) return CACTO_E_ARG;
+    if (reinterpret_cast<uintptr_t>(part) & 15) return CACTO_E_ALIGN;
+    const int64_t need = cacto_det_partials_floats(CACTO_DET_CRITIC_TC, B, p->ns, p->na, 0, 0);
+    if (need < 0 || part_floats < need) return CACTO_E_SIZE;
+  }
   TcWs ws;
   if (tc_ws_layout(static_cast<unsigned char*>(workspace), B, p->ns, p->na, &ws) > workspace_bytes) return CACTO_E_SIZE;
   cudaStream_t st = (cudaStream_t)stream;
@@ -1402,17 +1503,23 @@ extern "C" int cacto_critic_grad_tc(const cacto_sys_params* p, const float* crit
   memset(&BA, 0, sizeof(BA));
   BA.critic = critic_params; BA.w_S = w_S; BA.sobolev = sobolev ? 1 : 0; BA.mc = mc; BA.prtg = partial_rtg; BA.dVdx = dVdx; BA.done = done; BA.weights = weights;
   BA.V = V; BA.inv_B = inv_B; BA.rtg_out = rtg; BA.loss_out = loss; BA.grad = grad; BA.B = B;
-  const int grid = ntiles < sms ? ntiles : sms;
+  const int grid = det_grid<DET>(ntiles < sms ? ntiles : sms);
+  const size_t smem = sizeof(CriticSmemTc) + (DET ? TC_DET_SMEM : 0);
+  // DET: one partials region of `grid` slices per colsum kernel, in launch order (G, adjoint, B)
+  const int regions = sobolev ? 3 : 1;
+  auto region = [&](int r) { return DET ? part + (int64_t)r * grid * TC_DET_SLICE : grad; };
   if (sobolev) {
-    if (int e = tc_smem_attr(k_tc_critic_bwd<BWD_G>, sizeof(CriticSmemTc))) return e;
-    if (cudaError_t le_ = launch_tc(k_tc_critic_bwd<BWD_G>, dim3(grid), THREADS, sizeof(CriticSmemTc), st, *p, BA, ws, seq_critic_bwd(4), ntiles)) return (int)le_;
+    BA.grad = region(0);
+    if (int e = tc_smem_attr(k_tc_critic_bwd<BWD_G, DET>, smem)) return e;
+    if (cudaError_t le_ = launch_tc(k_tc_critic_bwd<BWD_G, DET>, dim3(grid), THREADS, smem, st, *p, BA, ws, seq_critic_bwd(4), ntiles)) return (int)le_;
     CACTO_LAUNCH_CHECK();
-    if (int e = tc_smem_attr(k_tc_critic_adj, sizeof(CriticSmemTc))) return e;
-    if (cudaError_t le_ = launch_tc(k_tc_critic_adj, dim3(grid), THREADS, sizeof(CriticSmemTc), st, *p, critic_params, grad, ws, seq_critic_fwd(), ntiles, B)) return (int)le_;
+    if (int e = tc_smem_attr(k_tc_critic_adj<DET>, smem)) return e;
+    if (cudaError_t le_ = launch_tc(k_tc_critic_adj<DET>, dim3(grid), THREADS, smem, st, *p, critic_params, region(1), ws, seq_critic_fwd(), ntiles, B)) return (int)le_;
     CACTO_LAUNCH_CHECK();
   }
-  if (int e = tc_smem_attr(k_tc_critic_bwd<BWD_B>, sizeof(CriticSmemTc))) return e;
-  if (cudaError_t le_ = launch_tc(k_tc_critic_bwd<BWD_B>, dim3(grid), THREADS, sizeof(CriticSmemTc), st, *p, BA, ws, seq_critic_bwd(3), ntiles)) return (int)le_;
+  BA.grad = region(regions - 1);
+  if (int e = tc_smem_attr(k_tc_critic_bwd<BWD_B, DET>, smem)) return e;
+  if (cudaError_t le_ = launch_tc(k_tc_critic_bwd<BWD_B, DET>, dim3(grid), THREADS, smem, st, *p, BA, ws, seq_critic_bwd(3), ntiles)) return (int)le_;
   CACTO_LAUNCH_CHECK();
 
   const CriticLayout CL(p->ns);
@@ -1433,21 +1540,38 @@ extern "C" int cacto_critic_grad_tc(const cacto_sys_params* p, const float* crit
     J.E[1] = wg_op(ws.DL, CWT, kofs(l), AM_DL);
     J.M = CL.in[l]; J.N = CL.out[l]; J.N_real = CL.out[l]; J.ld = CL.out[l]; J.ldn = 1; J.out = grad + CL.W[l];
   }
-  return launch_wgrad(WT, ws, sms, st);
+  if (int e = launch_wgrad(WT, ws, sms, st)) return e;
+  if (DET) {
+    if (cudaError_t le_ = launch_tc(k_tc_det_reduce, dim3((TC_DET_SLICE + 255) / 256), 256, 0, st, (const float*)part, regions, grid, 1, (int)p->ns,
+                                    (int)p->na, grad, loss)) return (int)le_;
+    CACTO_LAUNCH_CHECK();
+  }
+  return 0;
 }
 
-extern "C" int cacto_actor_grad_tc(const cacto_sys_params* p, const float* actor_params, const float* critic_params, const float* state,
+
+template <bool DET>
+static int actor_grad_tc(const cacto_sys_params* p, const float* actor_params, const float* critic_params, const float* state,
                                    const double* term, float inv_B, float* grad, float* actions, int64_t B, void* workspace, int64_t workspace_bytes,
-                                   void* stream) {
+                                   float* part, int64_t part_floats, void* stream) {
   if (!p) return CACTO_E_ARG;
   if (B < 0) return CACTO_E_SIZE;
   if (B == 0) return 0;
   if (!actor_params || !critic_params || !state || !term || !grad || !workspace) return CACTO_E_ARG;
   if ((reinterpret_cast<uintptr_t>(workspace) & 255) || (reinterpret_cast<uintptr_t>(grad) & 15)) return CACTO_E_ALIGN;
+  if (DET) {
+    if (!part) return CACTO_E_ARG;
+    if (reinterpret_cast<uintptr_t>(part) & 15) return CACTO_E_ALIGN;
+    const int64_t need = cacto_det_partials_floats(CACTO_DET_ACTOR_TC, B, p->ns, p->na, 0, 0);
+    if (need < 0 || part_floats < need) return CACTO_E_SIZE;
+  }
   TcWs ws;
   if (tc_ws_layout(static_cast<unsigned char*>(workspace), B, p->ns, p->na, &ws) > workspace_bytes) return CACTO_E_SIZE;
   cudaStream_t st = (cudaStream_t)stream;
-  const int ntiles = (int)ws.tiles, sms = num_sms(), grid = ntiles < sms ? ntiles : sms;
+  const int ntiles = (int)ws.tiles, sms = num_sms(), grid = det_grid<DET>(ntiles < sms ? ntiles : sms);
+  const size_t smem_c = sizeof(CriticSmemTc) + (DET ? TC_DET_SMEM : 0), smem_a = sizeof(ActorSmemTc) + (DET ? TC_DET_SMEM : 0);
+  // DET: one partials region of `grid` slices per colsum kernel, in launch order (GP, actor backward)
+  auto region = [&](int r) { return DET ? part + (int64_t)r * grid * TC_DET_SLICE : grad; };
 
   PrepTable PT;
   memset(&PT, 0, sizeof(PT));
@@ -1483,13 +1607,13 @@ extern "C" int cacto_actor_grad_tc(const cacto_sys_params* p, const float* actor
 
   BwdArgs BA;
   memset(&BA, 0, sizeof(BA));
-  BA.critic = critic_params; BA.inv_B = inv_B; BA.grad = grad; BA.B = B;
-  if (int e = tc_smem_attr(k_tc_critic_bwd<BWD_GP>, sizeof(CriticSmemTc))) return e;
-  if (cudaError_t le_ = launch_tc(k_tc_critic_bwd<BWD_GP>, dim3(grid), THREADS, sizeof(CriticSmemTc), st, *p, BA, ws, seq_critic_bwd(4), ntiles)) return (int)le_;
+  BA.critic = critic_params; BA.inv_B = inv_B; BA.grad = region(0); BA.B = B;
+  if (int e = tc_smem_attr(k_tc_critic_bwd<BWD_GP, DET>, smem_c)) return e;
+  if (cudaError_t le_ = launch_tc(k_tc_critic_bwd<BWD_GP, DET>, dim3(grid), THREADS, smem_c, st, *p, BA, ws, seq_critic_bwd(4), ntiles)) return (int)le_;
   CACTO_LAUNCH_CHECK();
 
-  if (int e = tc_smem_attr(k_tc_actor_bwd, sizeof(ActorSmemTc))) return e;
-  if (cudaError_t le_ = launch_tc(k_tc_actor_bwd, dim3(grid), THREADS, sizeof(ActorSmemTc), st, *p, grad, ws, seq_actor_bwd(), ntiles, B)) return (int)le_;
+  if (int e = tc_smem_attr(k_tc_actor_bwd<DET>, smem_a)) return e;
+  if (cudaError_t le_ = launch_tc(k_tc_actor_bwd<DET>, dim3(grid), THREADS, smem_a, st, *p, region(1), ws, seq_actor_bwd(), ntiles, B)) return (int)le_;
   CACTO_LAUNCH_CHECK();
 
   const ActorLayout AL(p->ns, p->na);
@@ -1511,5 +1635,41 @@ extern "C" int cacto_actor_grad_tc(const cacto_sys_params* p, const float* actor
     J.nterms = 1; J.X[0] = wg_op(ws.D3, 16, 0, AM_D3); J.E[0] = wg_op(ws.H2, ACTOR_H, 0, AM_H2);
     J.M = p->na; J.N = ACTOR_H; J.N_real = ACTOR_H; J.ld = 1; J.ldn = p->na; J.out = grad + AL.W3;
   }
-  return launch_wgrad(WT, ws, sms, st);
+  if (int e = launch_wgrad(WT, ws, sms, st)) return e;
+  if (DET) {
+    if (cudaError_t le_ = launch_tc(k_tc_det_reduce, dim3((TC_DET_SLICE + 255) / 256), 256, 0, st, (const float*)part, 2, grid, 0, (int)p->ns,
+                                    (int)p->na, grad, (float*)nullptr)) return (int)le_;
+    CACTO_LAUNCH_CHECK();
+  }
+  return 0;
 }
+
+extern "C" int cacto_critic_grad_tc(const cacto_sys_params* p, const float* critic_params, const float* target_params, float w_S, int mc,
+                                    const float* state, const float* state_next, const float* partial_rtg, const float* dVdx, const float* done,
+                                    const float* weights, float inv_B, float* grad, float* rtg, float* V, float* V_target_s, float* loss, int64_t B,
+                                    void* workspace, int64_t workspace_bytes, void* stream) {
+  return critic_grad_tc<false>(p, critic_params, target_params, w_S, mc, state, state_next, partial_rtg, dVdx, done, weights, inv_B, grad, rtg, V,
+                               V_target_s, loss, B, workspace, workspace_bytes, nullptr, 0, stream);
+}
+
+extern "C" int cacto_critic_grad_tc_det(const cacto_sys_params* p, const float* critic_params, const float* target_params, float w_S, int mc,
+                                        const float* state, const float* state_next, const float* partial_rtg, const float* dVdx, const float* done,
+                                        const float* weights, float inv_B, float* grad, float* rtg, float* V, float* V_target_s, float* loss, int64_t B,
+                                        void* workspace, int64_t workspace_bytes, float* partials, int64_t partials_floats, void* stream) {
+  return critic_grad_tc<true>(p, critic_params, target_params, w_S, mc, state, state_next, partial_rtg, dVdx, done, weights, inv_B, grad, rtg, V,
+                              V_target_s, loss, B, workspace, workspace_bytes, partials, partials_floats, stream);
+}
+
+extern "C" int cacto_actor_grad_tc(const cacto_sys_params* p, const float* actor_params, const float* critic_params, const float* state,
+                                   const double* term, float inv_B, float* grad, float* actions, int64_t B, void* workspace, int64_t workspace_bytes,
+                                   void* stream) {
+  return actor_grad_tc<false>(p, actor_params, critic_params, state, term, inv_B, grad, actions, B, workspace, workspace_bytes, nullptr, 0, stream);
+}
+
+extern "C" int cacto_actor_grad_tc_det(const cacto_sys_params* p, const float* actor_params, const float* critic_params, const float* state,
+                                       const double* term, float inv_B, float* grad, float* actions, int64_t B, void* workspace, int64_t workspace_bytes,
+                                       float* partials, int64_t partials_floats, void* stream) {
+  return actor_grad_tc<true>(p, actor_params, critic_params, state, term, inv_B, grad, actions, B, workspace, workspace_bytes, partials, partials_floats,
+                             stream);
+}
+

@@ -28,6 +28,7 @@ if int(ops.abi_version()) != 1:
 
 OP_NAMES = ('abi_version', 'dyn_step', 'dyn_derivative', 'dyn_augmented', 'ee_position', 'reward', 'rollout', 'actor_tc16_prepare', 'rollout_tc16',
             'rollout_width', 'actor_forward_width', 'actor_grad_width', 'actor_forward', 'critic_forward', 'critic_grad', 'actor_grad', 'update_tc_workspace_bytes', 'critic_grad_tc', 'actor_grad_tc',
+            'det_partials_floats', 'critic_grad_det', 'actor_grad_det', 'actor_grad_width_det', 'critic_grad_tc_det', 'actor_grad_tc_det',
             'adam_schedule', 'adam_schedule2', 'adam_step', 'transpose_params', 'segtree_update', 'segtree_sample', 'buffer_gather', 'rtg_window')
 
 

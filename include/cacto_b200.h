@@ -291,6 +291,49 @@ int cacto_actor_grad_tc(const cacto_sys_params* p, const float* actor_params, co
                         const double* term, float inv_B, float* grad, float* actions /* [B][na] or NULL */, int64_t B,
                         void* workspace, int64_t workspace_bytes, void* stream);
 
+/* ---- Deterministic N6 / N7 (NN(..., deterministic=True)): the contracts of cacto_critic_grad, cacto_actor_grad and
+ *      cacto_actor_grad_width on the same fused fp32 kernels, but with every cross-CTA and cross-warp float sum taken in a fixed
+ *      order, so that the same inputs give the same bits in grad, rtg, V, V_target_s and loss however the CTAs are scheduled.
+ *      Each CTA (one tile of samples) writes its sums into its own slice of `partials`; one reduce kernel then adds the slices
+ *      into grad in slice order, starting from 0.0f, and adds that into what grad holds (the accumulate-into-grad contract is
+ *      kept; loss, if not NULL, receives the summed loss the same way).  Results differ from the default entry points only in
+ *      summation order; they depend on the batch size (the tile size and the slice count follow it).
+ *      partials: caller-owned, 16-byte aligned, at least cacto_det_partials_floats(net, B, ns, na, nh1, nh2) floats, where net is
+ *      CACTO_DET_CRITIC, CACTO_DET_ACTOR (nh1, nh2 ignored) or CACTO_DET_ACTOR_WIDTH.  A slice holds the network's gradient block
+ *      plus one loss partial (rounded up to 4 floats); there are min(tiles, CACTO_DET_MAX_SLICES) slices, so the workspace stops
+ *      growing with B once the batch has more tiles than that (more tiles run as successive launches of at most
+ *      CACTO_DET_MAX_SLICES CTAs, CTA j of each adding into slice j).  Critic and actor calls that may run concurrently need
+ *      separate workspaces.  The size query returns CACTO_E_SIZE for out-of-range arguments.  No host synchronisation;
+ *      capturable.
+ *      cacto_critic_grad_tc_det / cacto_actor_grad_tc_det: the same for the tcgen05 engine (contracts of cacto_critic_grad_tc /
+ *      cacto_actor_grad_tc, same workspace).  Its weight matrices are already summed in a fixed order; the bias and head column
+ *      sums and the loss are summed per warp, then in warp order inside a CTA, and each CTA writes them into its own slice of
+ *      `partials` (net CACTO_DET_CRITIC_TC / CACTO_DET_ACTOR_TC: at most 3 / 2 regions of min(B / 128 tiles, CACTO_DET_MAX_SLICES)
+ *      slices of 648 floats, every entry written, so no clearing), which one reduce kernel adds into grad in slice order. */
+#define CACTO_DET_MAX_SLICES 296
+enum { CACTO_DET_CRITIC = 0, CACTO_DET_ACTOR = 1, CACTO_DET_ACTOR_WIDTH = 2, CACTO_DET_CRITIC_TC = 3, CACTO_DET_ACTOR_TC = 4 };
+int64_t cacto_det_partials_floats(int32_t net, int64_t B, int32_t ns, int32_t na, int32_t nh1, int32_t nh2);
+int cacto_critic_grad_det(const cacto_sys_params* p, const float* critic_params, const float* critic_params_T,
+                          const float* target_params, float w_S, int mc, const float* state, const float* state_next,
+                          const float* partial_rtg, const float* dVdx, const float* done, const float* weights,
+                          float inv_B, float* grad, float* rtg, float* V, float* V_target_s, float* loss,
+                          int64_t B, float* partials, int64_t partials_floats, void* stream);
+int cacto_actor_grad_det(const cacto_sys_params* p, const float* actor_params, const float* actor_params_T,
+                         const float* critic_params, const float* critic_params_T, const float* state,
+                         const double* term, float inv_B, float* grad, float* actions /* [B][na] or NULL */,
+                         int64_t B, float* partials, int64_t partials_floats, void* stream);
+int cacto_actor_grad_width_det(const cacto_sys_params* p, const float* actor_params, int32_t nh1, int32_t nh2, const float* critic_params,
+                               const float* critic_params_T, const float* state, const double* term, float inv_B, float* grad,
+                               float* actions /* [B][na] or NULL */, int64_t B, float* partials, int64_t partials_floats, void* stream);
+int cacto_critic_grad_tc_det(const cacto_sys_params* p, const float* critic_params, const float* target_params, float w_S, int mc,
+                             const float* state, const float* state_next, const float* partial_rtg, const float* dVdx,
+                             const float* done, const float* weights, float inv_B, float* grad, float* rtg, float* V,
+                             float* V_target_s, float* loss /* [1], accumulated, or NULL */, int64_t B, void* workspace,
+                             int64_t workspace_bytes, float* partials, int64_t partials_floats, void* stream);
+int cacto_actor_grad_tc_det(const cacto_sys_params* p, const float* actor_params, const float* critic_params, const float* state,
+                            const double* term, float inv_B, float* grad, float* actions /* [B][na] or NULL */, int64_t B,
+                            void* workspace, int64_t workspace_bytes, float* partials, int64_t partials_floats, void* stream);
+
 /* ---- N8/N9: tf.keras Adam step (RL.py:105,109; TF 2.11: m += (g-m)(1-b1), v += (g^2-v)(1-b2),
  *      p -= alpha_t m / (sqrt(v) + eps)) fused with the optional Polyak target update (RL.py:113-118:
  *      target = tau p + (1-tau) target), the refresh of the transposed copy and the zeroing of `grad`.
