@@ -5,7 +5,10 @@
 //     a' = 2^p a = a_hi + a_lo,  w' = 2^s w = w_hi + w_lo,   a' w' ~= a_hi w_hi + a_hi w_lo + a_lo w_hi   (fp32 accumulation in TMEM)
 // with power-of-two scales (exact): per weight matrix from max|W| (prepare kernel), per ROW of the activation tile from a bound
 // on the row's magnitude (the thread that owns the row knows it), so that no operand leaves the fp16 range however the
-// network was trained.  Relative error of a product ~2^-21, the class of the fp32 FMA kernels within the 1e-4 parity gate.
+// network was trained.  Relative error of a product ~2^-21; a CPU emulation of the split with these scales stays within the fp32
+// error per layer on trained networks (tests/test_trained_nets.py).  The engine as a whole does not: on the reference's trained
+// double-integrator actor its actions are ~35x and its dW3 ~22x the fp32 oracle's distance from fp64 (dW3 1.07e-4, just past the
+// 1e-4 parity gate; tests/test_gpu_trained_nets.py K_TC).  The source of that excess is not located yet.
 //
 // Kernel skeleton ("chain kernel"): a persistent CTA walks a list of jobs (one 128-row tile each); per job a chain of layers
 //     [epilogue threads write the A image of layer l] -> a_full -> [issuer: UMMAs over the K-chunks of W_l] -> d_full ->

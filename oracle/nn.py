@@ -201,13 +201,14 @@ def polyak(target, source, tau):
         a[...] = b * f(tau) + a * f(1 - tau)
 
 
-def update(critic, target, actor, opt_c, opt_a, conf, w_S, env, batch):
+def update(critic, target, actor, opt_c, opt_a, conf, w_S, env, batch, dtype=torch.float32):
     """One RL_AC.update + update_target (RL.py:101-111,134-135).  ``batch`` =
-    (state, partial_rtg, state_next, dVdx, d, term, weights).  In-place on the parameter lists."""
+    (state, partial_rtg, state_next, dVdx, d, term, weights).  In-place on the parameter lists.  ``dtype`` is the precision of
+    the gradients (as in critic_grad / actor_grad); Adam and Polyak stay in float32 as in the reference."""
     state, partial_rtg, state_next, dVdx, d, term, weights = batch
-    cg, rtg, V, Vt, loss = critic_grad(critic, target, conf, w_S, state, state_next, partial_rtg, dVdx, d, weights)
+    cg, rtg, V, Vt, loss = critic_grad(critic, target, conf, w_S, state, state_next, partial_rtg, dVdx, d, weights, dtype=dtype)
     opt_c.apply_gradients(critic, cg)
-    ag, actions, s_next, dQ = actor_grad(actor, critic, conf, env, state, term)
+    ag, actions, s_next, dQ = actor_grad(actor, critic, conf, env, state, term, dtype=dtype)
     opt_a.apply_gradients(actor, ag)
     if not conf.MC:
         polyak(target, critic, conf.UPDATE_RATE)
